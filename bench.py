@@ -28,6 +28,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 WORKLOADS = {
     # name: (sites, haplotypes, queries per GPU per step)
@@ -69,6 +70,8 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extract", action="store_true", help="skip the configs[4] extraction inside the default run")
     ap.add_argument("--no-runs", action="store_true", help="skip the run-length workload inside the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's share) to DIR/<name>.npy, at most 64 MB in all")
     return ap.parse_args()
 
 
@@ -205,6 +208,30 @@ def run_reference(args, rank, world):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every device tensor of `arrays` as out_dir/<name>.npy in float64, which holds every value the timed
+    paths return exactly. The inputs are the same from run to run, so two builds can be compared array by array. A tensor
+    larger than its share of DUMP_BYTES is written as a fixed, seeded sample of its rows in ascending order, and the row
+    numbers of the sample as <name>_rows.npy."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        n = t.shape[0]
+        row_bytes = 8 * (t.numel() // n if n else 1)
+        if n * row_bytes + 1024 <= share:
+            host = t.cpu().numpy()
+        else:
+            rows = np.sort(np.random.default_rng(SEED).choice(n, size=(share - 2048) // (row_bytes + 8), replace=False))
+            host = t[torch.from_numpy(rows).to(t.device)].cpu().numpy()
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), host.astype(np.float64))
+    log(f"[bench] outputs of the last timed step written to {out_dir}: {', '.join(arrays)}")
 
 
 def resolve_workload(args):
@@ -370,6 +397,8 @@ def main():
 
     total_ms, step_ms, clocks, launches = timed_steps(step, args.steps, args.warmup)
     value = Q * world * args.steps / (total_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"states": d_out})  # (node, start, end) of every query
 
     # size-independent parity properties on the full batch (every sampled pattern occurs; state.node = last node)
     ok = bool(torch.all(d_out[:, 2] > d_out[:, 1]).item()) and bool(torch.equal(d_out[:, 0], d_pat[:, K_LEN - 1]))
@@ -778,6 +807,8 @@ def bench_extract(args, index, image, sites, haplotypes, rank, world, local_rank
     t1 = time.time()
     total_ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop(t0, t1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"nodes": nodes, "lengths": lens})
     assert bool(torch.all(lens == length).item())
     from synth import synth
     first = nodes[:length].cpu().numpy().view(np.uint64)
@@ -852,6 +883,8 @@ def bench_extract_dna(args, index, image, sites, haplotypes, rank, world, local_
     t1 = time.time()
     total_ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop(t0, t1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"dna": out, "lengths": got})
     assert bool(torch.all(got == lens).item())
     launches = gb.kernel_launches() - launches0
     # the same walks without the byte copy (label ranges and lengths only, one-ended), for the cost split

@@ -11,6 +11,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 from typing import Optional, Sequence
 
 import numpy as np
@@ -39,14 +40,24 @@ class BDState(C.Structure):
     _fields_ = [("forward", State), ("reverse", State)]
 
 
+_NATIVE_DIR = None
+
+
 def build(native: bool = False, force: bool = False) -> str:
-    """Compile the oracle with the committed Makefile; returns the .so path."""
-    out = "libgbwt_oracle_native.so" if native else "libgbwt_oracle.so"
-    path = os.path.join(_HERE, out)
+    """Compile the oracle with the committed Makefile; returns the .so path. The -march=native copy is built for the host
+    that runs it, so it goes to a temporary directory of this process (removed at exit), never into the tree: the
+    benchmark uses it and may run from a read-only tree."""
+    global _NATIVE_DIR
+    if native:
+        if _NATIVE_DIR is None:
+            _NATIVE_DIR = tempfile.TemporaryDirectory(prefix="gbwt_oracle_")
+        path = os.path.join(_NATIVE_DIR.name, "libgbwt_oracle_native.so")
+    else:
+        path = os.path.join(_HERE, "libgbwt_oracle.so")
     src = [os.path.join(_HERE, f) for f in ("gbwt_oracle.c", "gbwt_oracle.h", "Makefile")]
     stale = (not os.path.exists(path)) or any(os.path.getmtime(s) > os.path.getmtime(path) for s in src)
     if force or stale:
-        cmd = ["make", "-C", _HERE, "-B", f"OUT={out}"]
+        cmd = ["make", "-C", _HERE, "-B", f"OUT={path}"]
         if native:
             cmd.append("MARCH=native")
         subprocess.run(cmd, check=True, capture_output=True)
