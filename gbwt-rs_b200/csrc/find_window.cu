@@ -325,7 +325,9 @@ __device__ __forceinline__ void window_extend(const Staged& st, uint32_t slot, u
             const uint32_t total = h.y & 0xFFFFu, kind = h.y >> 16;
             const uint32_t s = start < total ? start : total, e = end < total ? end : total;
             if (x1 == NODE_OUTSIDE) { status = QUERY_DEFER; break; }
-            if (s >= e) { status = QUERY_NONE; break; }  // Record::follow on an empty range
+            // Record::follow on an empty range; a record of 0xFFFF positions or more is staged with total 0 (KIND_DEFER), and
+            // its range is only empty here because it was not staged
+            if (s >= e) { status = kind == KIND_DEFER ? QUERY_DEFER : QUERY_NONE; break; }
             const uint32_t b = x1 == (h.x >> 16) ? 1u : 0u;
             uint32_t rs = s, re = e;
             if (kind < KIND_WIDE) {
@@ -979,7 +981,7 @@ __device__ __forceinline__ uint32_t bd_window_extend(const Staged& st, uint32_t 
         if (x1 == NODE_OUTSIDE) { status = QUERY_DEFER; break; }
         const uint32_t total = h.y & 0xFFFFu, kind = h.y >> 16;
         const uint32_t s = a_start < total ? a_start : total, e = a_end < total ? a_end : total;
-        if (s >= e) { status = QUERY_NONE; break; }
+        if (s >= e) { status = kind == KIND_DEFER ? QUERY_DEFER : QUERY_NONE; break; }  // (as in window_extend)
         const uint32_t t0 = h.x & 0xFFFFu, t1 = h.x >> 16;
         uint32_t b = 0, rs = s, re = e, moved = 0;
         if (kind < KIND_WIDE) {

@@ -6,6 +6,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <type_traits>
+#include <vector>
 #ifdef _OPENMP
 #include <omp.h>
 #endif
@@ -101,12 +102,19 @@ Plan plan_record(const uint8_t* bytes, uint64_t len, int policy, const Checkpoin
     if (!rd.varint(pl.sigma)) { pl.status = GBWT_B200_E_INVALID_DATA; return pl; }
     if (pl.sigma == 0) return pl;  // decompress_edges: sigma == 0 -> None (src/bwt.rs:381)
     if (pl.sigma > 0xFFFFFFFFull) { pl.status = GBWT_B200_E_RANGE; return pl; }
+    // room[b] = how many positions edge b can still send before offset_b + rank passes 2^32 - 1: the kernels add edge
+    // offsets and ranks in 32 bits. A consistent index never runs out (offset_b + count_b <= the target's length < 2^32).
+    // (one buffer per thread, reused from record to record; every edge takes at least two bytes of the record)
+    if (pl.sigma > (len - rd.at) / 2) { pl.status = GBWT_B200_E_INVALID_DATA; return pl; }
+    thread_local std::vector<uint64_t> room;
+    room.resize(pl.sigma);
     uint64_t node = 0;
     for (uint64_t i = 0; i < pl.sigma; i++) {
         uint64_t delta, off;
         if (!rd.varint(delta) || !rd.varint(off)) { pl.status = GBWT_B200_E_INVALID_DATA; return pl; }
         node += delta;
         if (node > 0xFFFFFFFFull || off > 0xFFFFFFFFull) { pl.status = GBWT_B200_E_RANGE; return pl; }
+        room[i] = 0xFFFFFFFFull - off;
     }
     pl.header_end = rd.at;
     rd.begin_runs(pl.sigma);
@@ -116,6 +124,8 @@ Plan plan_record(const uint8_t* bytes, uint64_t len, int policy, const Checkpoin
         if (value >= pl.sigma) { pl.status = GBWT_B200_E_INVALID_DATA; return pl; }
         // a run longer than the 32-bit layout (a crafted length near 2^64 would wrap the sums below)
         if (rl == 0 || rl > 0xFFFFFFFFull) { pl.status = GBWT_B200_E_RANGE; return pl; }
+        if (rl > room[value]) { pl.status = GBWT_B200_E_RANGE; return pl; }
+        room[value] -= rl;
         pl.total += rl;
         if (value < 2) pl.count01[value] += rl;
         pl.runs++;

@@ -8,9 +8,12 @@
  *
  * Conventions
  *  - All integers are 64-bit like the crate's `usize`; nothing is truncated at the boundary. The device
- *    layout stores node ids, offsets and record lengths in 32 bits, so an index whose alphabet size or
- *    any record length reaches 2^32 is rejected at load with GBWT_B200_E_RANGE (it could not fit a
- *    B200's HBM either: one 32-byte record descriptor per node).
+ *    layout stores node ids, offsets and record lengths in 32 bits, so an index whose alphabet size
+ *    exceeds 2^32 (a node id above 2^32 - 1) or whose record length reaches 2^32 is rejected at load
+ *    with GBWT_B200_E_RANGE (it could not fit a B200's HBM either: one 32-byte record descriptor per
+ *    node). So is an index in which some edge b of a record has offset_b + count_b > 2^32 - 1, count_b
+ *    being the number of the record's positions with symbol b: the kernels add edge offsets and ranks in
+ *    32 bits. A consistent index never has one (offset_b + count_b is at most the length of b's record).
  *  - `Option::None` is encoded in-band: a SearchState with start >= end is None and is canonicalised to
  *    {0,0,0} (the reference guarantees Some => non-empty range, src/bwt.rs:615, 448); a None Pos is {0,0}
  *    (a Some Pos never has node == ENDMARKER, src/gbwt.rs:213-219, src/bwt.rs:485-486).
