@@ -27,18 +27,22 @@ ENDMARKER = 0  # gbwt-rs src/lib.rs:59
 STATE_DTYPE = np.dtype([("node", "<u8"), ("start", "<u8"), ("end", "<u8")])
 BDSTATE_DTYPE = np.dtype([("forward", STATE_DTYPE), ("reverse", STATE_DTYPE)])
 POS_DTYPE = np.dtype([("node", "<u8"), ("offset", "<u8")])
+OCCURRENCE_DTYPE = np.dtype([("sequence", "<u8"), ("index", "<u8")])  # gbwt_b200_occurrence
 
 LAYOUT_AUTO, LAYOUT_RUNS = 0, 1
 LAYOUT_CHECKPOINTS, LAYOUT_NO_CHECKPOINTS = 0x100, 0x200
+LAYOUT_LOCATE = 0x400  # locate samples (GBWT.locate); the `locate=True` keyword of load / from_bytes / from_parts
 _LAYOUTS = {"auto": LAYOUT_AUTO, "runs": LAYOUT_RUNS, 0: LAYOUT_AUTO, 1: LAYOUT_RUNS}
 
 
-def _policy(layout, checkpoints) -> int:
-    """Layout policy word of the C ABI: body layout + the checkpoint flag (None = the library's default by size)."""
+def _policy(layout, checkpoints, locate=False) -> int:
+    """Layout policy word of the C ABI: body layout + the checkpoint flag (None = the library's default by size) + the
+    locate-sample flag."""
     flag = 0 if checkpoints is None else (LAYOUT_CHECKPOINTS if checkpoints else LAYOUT_NO_CHECKPOINTS)
-    return _LAYOUTS[layout] | flag
+    return _LAYOUTS[layout] | flag | (LAYOUT_LOCATE if locate else 0)
 
 OK, E_INVALID_DATA, E_IO, E_RANGE, E_NOT_BIDIRECTIONAL, E_CUDA, E_ARGUMENT, E_NO_DEVICE = range(8)
+E_NO_GRAPH, E_NO_SAMPLES = 8, 9
 _U64MAX = np.uint64(2**64 - 1)
 
 
@@ -77,6 +81,11 @@ def _load_library() -> C.CDLL:
         "gbwt_b200_device_bytes": (u64, [p, p]),
         "gbwt_b200_window_info": (None, [p, p]),
         "gbwt_b200_checkpoint_info": (None, [p, p]),
+        "gbwt_b200_locate_info": (None, [p, p]),
+        "gbwt_b200_locate": (i, [p, p, sz, p]),
+        "gbwt_b200_locate_states": (i, [p, p, sz, p, p, p]),
+        "gbwt_b200_locate_device": (i, [p, p, sz, p, p]),
+        "gbwt_b200_locate_states_device": (i, [p, p, sz, p, p, p, p]),
         "gbwt_b200_find": (i, [p, p, sz, p]),
         "gbwt_b200_extend": (i, [p, p, p, sz, p]),
         "gbwt_b200_find_extend": (i, [p, p, sz, sz, p]),
@@ -236,27 +245,27 @@ class GBWT:
             raise GBWTError(rc, msg)
 
     @classmethod
-    def load(cls, path, device: int = 0, layout="auto", checkpoints=None) -> "GBWT":
+    def load(cls, path, device: int = 0, layout="auto", checkpoints=None, locate=False) -> "GBWT":
         h = C.c_void_p()
-        cls._check(_lib.gbwt_b200_index_load_file(os.fsencode(path), device, _policy(layout, checkpoints), C.byref(h)))
+        cls._check(_lib.gbwt_b200_index_load_file(os.fsencode(path), device, _policy(layout, checkpoints, locate), C.byref(h)))
         return cls(h.value)
 
     @classmethod
-    def from_bytes(cls, image, device: int = 0, layout="auto", checkpoints=None) -> "GBWT":
+    def from_bytes(cls, image, device: int = 0, layout="auto", checkpoints=None, locate=False) -> "GBWT":
         arr = image if isinstance(image, np.ndarray) else np.frombuffer(image, dtype=np.uint8)
         arr = np.ascontiguousarray(arr)
         h = C.c_void_p()
-        cls._check(_lib.gbwt_b200_index_from_bytes(_ptr(arr), arr.nbytes, device, _policy(layout, checkpoints), C.byref(h)))
+        cls._check(_lib.gbwt_b200_index_from_bytes(_ptr(arr), arr.nbytes, device, _policy(layout, checkpoints, locate), C.byref(h)))
         return cls(h.value)
 
     @classmethod
     def from_parts(cls, sequences, size, offset, alphabet_size, flags, bwt_bytes, record_starts, device: int = 0,
-                   layout="auto") -> "GBWT":
+                   layout="auto", locate=False) -> "GBWT":
         data = np.ascontiguousarray(np.frombuffer(bytes(bwt_bytes), dtype=np.uint8))
         starts = _u64(record_starts)
         h = C.c_void_p()
         cls._check(_lib.gbwt_b200_index_from_parts(sequences, size, offset, alphabet_size, flags, _ptr(data), data.nbytes,
-                                                   _ptr(starts), len(starts), device, _LAYOUTS[layout], C.byref(h)))
+                                                   _ptr(starts), len(starts), device, _policy(layout, None, locate), C.byref(h)))
         return cls(h.value)
 
     def attach_graph(self, label_starts, label_bytes) -> "GBWT":
@@ -496,6 +505,55 @@ class GBWT:
             return None
         _, nodes, _ = self.extract(np.array([seq_id], dtype=np.uint64))
         return iter(int(x) for x in nodes)
+
+    # -- locate: which sequences, and where (beyond the crate; the C++ GBWT's locate is the model, gbwt_b200.h) --
+    def locate(self, what):
+        """A Pos: (sequence, index) of the position -- node number `index` of GBWT::sequence(sequence) -- or None where there
+        is no such position. A SearchState: the list of (sequence, index) of its positions in offset order (empty for None).
+        The C++ GBWT's locate(state) is sorted(set(s for s, _ in ...)). Needs an index created with locate=True."""
+        if isinstance(what, Pos):
+            r = self.locate_positions(np.array([(what.node, what.offset)], dtype=POS_DTYPE))[0]
+            return None if r["sequence"] == _U64MAX else (int(r["sequence"]), int(r["index"]))
+        if isinstance(what, SearchState):
+            _, occ = self.locate_states(np.array([_state_rec(what)], dtype=STATE_DTYPE))
+            return [(int(o["sequence"]), int(o["index"])) for o in occ]
+        if what is None:
+            return []
+        raise TypeError("locate takes a Pos or a SearchState")
+
+    def locate_positions(self, positions) -> np.ndarray:
+        """locate for many positions: a structured array of (sequence, index), UINT64_MAX in both where there is none."""
+        positions = np.ascontiguousarray(positions, dtype=POS_DTYPE)
+        out = np.zeros(len(positions), OCCURRENCE_DTYPE)
+        self._check(_lib.gbwt_b200_locate(self._h, _ptr(positions), len(positions), _ptr(out)))
+        return out
+
+    def locate_states(self, states):
+        """The occurrences of many search states: (offsets, occurrences), those of state i at occurrences[offsets[i]:offsets[i+1]],
+        in offset order (shaped like extract)."""
+        states = np.ascontiguousarray(states, dtype=STATE_DTYPE)
+        n = len(states)
+        sizes = np.where(states["end"] > states["start"], states["end"] - states["start"], np.uint64(0)).astype(np.uint64)
+        offsets = np.zeros(n + 1, np.uint64)
+        np.cumsum(sizes, out=offsets[1:])
+        out = np.zeros(int(offsets[-1]), OCCURRENCE_DTYPE)
+        counts = np.zeros(n, np.uint64)
+        self._check(_lib.gbwt_b200_locate_states(self._h, _ptr(states), n, _ptr(offsets), _ptr(out), _ptr(counts)))
+        assert np.array_equal(counts, sizes)
+        return offsets, out
+
+    def locate_device(self, d_positions: int, n: int, d_out: int, stream: int = 0):
+        self._check(_lib.gbwt_b200_locate_device(self._h, d_positions, n, d_out, stream))
+
+    def locate_states_device(self, d_states: int, n: int, d_out_offsets: int, d_out: int, d_counts: int = 0, stream: int = 0):
+        self._check(_lib.gbwt_b200_locate_states_device(self._h, d_states, n, d_out_offsets or None, d_out or None, d_counts or None, stream))
+
+    def locate_info(self) -> dict:
+        """Locate samples (gbwt_b200_locate_info); lf_steps is only counted with GBWT_B200_LOCATE_STATS=1."""
+        raw = np.zeros(6, dtype=np.uint64)
+        _lib.gbwt_b200_locate_info(self._h, _ptr(raw))
+        keys = ("present", "interval", "samples", "bytes", "build_us", "lf_steps")
+        return {k: int(v) for k, v in zip(keys, raw)}
 
     # -- node sequences and DNA-level extraction (GBZ files; src/gbz.rs:286-306, src/bin/gbz-extract.rs:173-189) --
     def has_graph(self) -> bool: return bool(_lib.gbwt_b200_has_graph(self._h))

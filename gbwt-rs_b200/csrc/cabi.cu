@@ -21,6 +21,7 @@
 #include "kernels.cuh"
 #include "layout_builder.h"
 #include "layout_writer.h"
+#include "locate.h"
 #include "sds_loader.h"
 
 using namespace gbwt_b200;
@@ -65,6 +66,13 @@ struct gbwt_b200_index {
     uint64_t bytes[4] = {0, 0, 0, 0};
     uint64_t format_counts[FMT_COUNT] = {0, 0, 0, 0, 0, 0, 0};
     uint64_t checkpointed_records = 0;
+    // Locate samples (GBWT_B200_LAYOUT_LOCATE; kernels.cuh k_build_locate, locate.cu): built once at creation.
+    void* d_locate_first = nullptr;    // u32 [records + 1]
+    void* d_locate_samples = nullptr;  // LocateSample [locate_samples]
+    bool locate_ok = false;
+    uint32_t locate_shift = 0;
+    uint64_t locate_samples = 0, locate_bytes = 0, locate_build_us = 0;
+    mutable std::atomic<uint64_t> locate_steps{0};  // GBWT_B200_LOCATE_STATS=1: LF steps of the locate walks
     Carried carried;  // tags, DA samples, metadata, Graph section: host-side, written back by serialize
 };
 
@@ -844,6 +852,59 @@ int attach_graph(gbwt_b200_index* ix, const uint64_t* starts, uint64_t sequences
     return GBWT_B200_OK;
 }
 
+int check_samples(const gbwt_b200_index* ix) {
+    if (!ix->locate_ok) return fail(GBWT_B200_E_NO_SAMPLES, "the index was created without locate samples (GBWT_B200_LAYOUT_LOCATE)");
+    return GBWT_B200_OK;
+}
+
+LocateView locate_view(const gbwt_b200_index* ix) {
+    LocateView lv;
+    lv.first = static_cast<const uint32_t*>(ix->d_locate_first);
+    lv.samples = static_cast<const LocateSample*>(ix->d_locate_samples);
+    // a walk meets a sample within 2^shift + 32 steps on a consistent index; the slack and walk_limit end it on a damaged one
+    lv.max_steps = std::min<uint64_t>((uint64_t(1) << ix->locate_shift) + 64, ix->view.walk_limit);
+    return lv;
+}
+
+// Runs `launch(steps)` on stream s; with GBWT_B200_LOCATE_STATS=1 it hands a device counter to the kernels, waits for the
+// stream and adds the LF steps they counted to the index's total.
+template <class Launch>
+int with_locate_stats(const gbwt_b200_index* ix, cudaStream_t s, Launch launch) {
+    if (env_int("GBWT_B200_LOCATE_STATS", 0) == 0) return launch(static_cast<unsigned long long*>(nullptr));
+    unsigned long long* steps = nullptr;
+    CUDA_TRY(cudaMallocAsync(reinterpret_cast<void**>(&steps), sizeof(unsigned long long), s));
+    CUDA_TRY(cudaMemsetAsync(steps, 0, sizeof(unsigned long long), s));
+    int rc = launch(steps);
+    unsigned long long host = 0;
+    if (rc == GBWT_B200_OK) {
+        cudaError_t e = cudaMemcpyAsync(&host, steps, sizeof(host), cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) rc = cuda_fail(e, "locate step counter");
+        else ix->locate_steps.fetch_add(host);
+    }
+    cudaFreeAsync(steps, s);
+    return rc;
+}
+
+int launch_locate_positions(const gbwt_b200_index* ix, const gbwt_b200_pos* pos, size_t n, gbwt_b200_occurrence* out, cudaStream_t s) {
+    if (n == 0) return GBWT_B200_OK;
+    return with_locate_stats(ix, s, [&](unsigned long long* steps) {
+        cudaError_t e = launch_locate(ix->view, locate_view(ix), pos, n, out, steps, ix->sm_count, s);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        return e == cudaSuccess ? GBWT_B200_OK : cuda_fail(e, "k_locate");
+    });
+}
+
+int launch_locate_state_batch(const gbwt_b200_index* ix, const gbwt_b200_state* states, size_t n, const uint64_t* out_offsets, uint64_t base,
+                              gbwt_b200_occurrence* out, uint64_t* counts, cudaStream_t s) {
+    if (n == 0) return GBWT_B200_OK;
+    return with_locate_stats(ix, s, [&](unsigned long long* steps) {
+        cudaError_t e = launch_locate_states(ix->view, locate_view(ix), states, n, out_offsets, base, out, counts, steps, ix->sm_count, s);
+        g_launches.fetch_add(out != nullptr ? 4 : 1, std::memory_order_relaxed);
+        return e == cudaSuccess ? GBWT_B200_OK : cuda_fail(e, "k_locate_states");
+    });
+}
+
 int check_graph(const gbwt_b200_index* ix) {
     if (!ix->has_graph) return fail(GBWT_B200_E_NO_GRAPH, "the index was not loaded from a GBZ file: no node sequences");
     return GBWT_B200_OK;
@@ -943,6 +1004,70 @@ int build_checkpoints(gbwt_b200_index* ix) {
     return GBWT_B200_OK;
 }
 
+// Locate samples: one walk over every sequence emits a sample at every 2^shift-th node (the first flush at or after it) and
+// at its last node (LocateSink), and locate.cu sorts them by BWT position. Default interval 2^10 (the C++ GBWT's sample
+// interval); GBWT_B200_LOCATE_SHIFT (0 .. 20) overrides it. The flag was asked for, so anything that keeps the table from
+// being built fails the creation.
+int build_locate(gbwt_b200_index* ix) {
+    const IndexView& v = ix->view;
+    if (v.sequences > 0xFFFFFFFFull) return fail(GBWT_B200_E_RANGE, "locate samples hold 32-bit sequence ids");
+    const uint32_t shift = static_cast<uint32_t>(std::min(20, std::max(0, env_int("GBWT_B200_LOCATE_SHIFT", 10))));
+    // at most one sample per multiple of the interval and one at the last node of every sequence (+ slack for the flushes)
+    const uint64_t cap = (v.walk_limit >> shift) + 2 * v.sequences + 1024;
+    cudaStream_t s = nullptr;
+    cudaEvent_t e0, e1;
+    CUDA_TRY(cudaEventCreate(&e0)); CUDA_TRY(cudaEventCreate(&e1));
+    uint64_t* keys = nullptr;
+    LocateSample* pool = nullptr;
+    unsigned long long* used_dev = nullptr;
+    uint32_t* first = nullptr;
+    LocateSample* table = nullptr;
+    auto cleanup = [&]() { cudaFree(keys); cudaFree(pool); cudaFree(used_dev); cudaEventDestroy(e0); cudaEventDestroy(e1); };
+    auto give_up = [&](int rc) { cleanup(); cudaFree(first); cudaFree(table); return rc; };
+    CUDA_TRY(cudaEventRecord(e0, s));
+    if (cudaMalloc(reinterpret_cast<void**>(&keys), cap * sizeof(uint64_t)) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&pool), cap * sizeof(LocateSample)) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&used_dev), sizeof(unsigned long long)) != cudaSuccess ||
+        cudaMemset(used_dev, 0, sizeof(unsigned long long)) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&first), (v.records + 1) * sizeof(uint32_t)) != cudaSuccess)
+        return give_up(cuda_fail(cudaGetLastError(), "cudaMalloc(locate samples)"));
+    int rc = GBWT_B200_OK;
+    if (shift >= 5) {
+        const int block = 128;
+        const unsigned ctas = static_cast<unsigned>(std::min<uint64_t>((v.sequences * 32 + block - 1) / block, uint64_t(1) << 20));
+        const uint32_t ahead = static_cast<uint32_t>(std::max(0, env_int("GBWT_B200_EXTRACT_AHEAD", 48)));
+        if (v.sequences > 0) {
+            if (v.edges_valid) k_build_locate<false><<<ctas, block, 0, s>>>(v, shift, keys, pool, used_dev, cap, ahead);
+            else k_build_locate<true><<<ctas, block, 0, s>>>(v, shift, keys, pool, used_dev, cap, ahead);
+        }
+    } else if (v.sequences > 0) {
+        k_build_locate_lanes<<<grid_for(ix, v.sequences), BLOCK_THREADS, 0, s>>>(v, shift, keys, pool, used_dev, cap);
+    }
+    rc = launch_done("k_build_locate");
+    unsigned long long used = 0;
+    if (rc == GBWT_B200_OK && cudaMemcpy(&used, used_dev, sizeof(used), cudaMemcpyDeviceToHost) != cudaSuccess)
+        rc = cuda_fail(cudaGetLastError(), "k_build_locate");
+    if (rc != GBWT_B200_OK) return give_up(rc);
+    if (used > 0xFFFFFFFFull) return give_up(fail(GBWT_B200_E_RANGE, "more than 2^32 - 1 locate samples (raise GBWT_B200_LOCATE_SHIFT)"));
+    // (only a damaged index, whose walks run to walk_limit, can emit more samples than the pool holds)
+    if (used > cap) return give_up(fail(GBWT_B200_E_INVALID_DATA, "locate samples: the sequences are longer than the index"));
+    if (cudaMalloc(reinterpret_cast<void**>(&table), std::max<size_t>(256, used * sizeof(LocateSample))) != cudaSuccess)
+        return give_up(cuda_fail(cudaGetLastError(), "cudaMalloc(locate table)"));
+    cudaError_t e = locate_sort_samples(keys, pool, used, v.records, table, first, ix->sm_count, s);
+    g_launches.fetch_add(2, std::memory_order_relaxed);
+    if (e == cudaSuccess) e = cudaEventRecord(e1, s);
+    if (e == cudaSuccess) e = cudaEventSynchronize(e1);
+    if (e != cudaSuccess) return give_up(cuda_fail(e, "locate sample sort"));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, e0, e1);
+    cleanup();
+    ix->d_locate_first = first; ix->d_locate_samples = table;
+    ix->locate_ok = true; ix->locate_shift = shift; ix->locate_samples = used;
+    ix->locate_bytes = used * sizeof(LocateSample) + (v.records + 1) * sizeof(uint32_t);
+    ix->locate_build_us = static_cast<uint64_t>(ms * 1000.0f);
+    return GBWT_B200_OK;
+}
+
 int create_index(const ParsedGBWT& parsed, int device, int policy, gbwt_b200_index** out) {
     if (out == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null output handle");
     *out = nullptr;
@@ -953,7 +1078,8 @@ int create_index(const ParsedGBWT& parsed, int device, int policy, gbwt_b200_ind
     }
     if (device < 0 || device >= count) return fail(GBWT_B200_E_ARGUMENT, "invalid device ordinal");
     const int checkpoint_policy = policy & (GBWT_B200_LAYOUT_CHECKPOINTS | GBWT_B200_LAYOUT_NO_CHECKPOINTS);
-    policy &= ~(GBWT_B200_LAYOUT_CHECKPOINTS | GBWT_B200_LAYOUT_NO_CHECKPOINTS);
+    const bool want_locate = (policy & GBWT_B200_LAYOUT_LOCATE) != 0;
+    policy &= ~(GBWT_B200_LAYOUT_CHECKPOINTS | GBWT_B200_LAYOUT_NO_CHECKPOINTS | GBWT_B200_LAYOUT_LOCATE);
     HostLayout layout;
     std::string err;
     int rc = build_layout(parsed, policy, layout, err);
@@ -1047,6 +1173,10 @@ int create_index(const ParsedGBWT& parsed, int device, int policy, gbwt_b200_ind
             if (rc != GBWT_B200_OK) { gbwt_b200_index_destroy(ix); return rc; }
             build_dna_checkpoints(ix);
         }
+    }
+    if (want_locate) {
+        rc = build_locate(ix);
+        if (rc != GBWT_B200_OK) { gbwt_b200_index_destroy(ix); return rc; }
     }
     *out = ix;
     return GBWT_B200_OK;
@@ -1175,7 +1305,7 @@ static int save_index(const gbwt_b200_index* ix, bool gbz, const char* path) {
 namespace {
 
 constexpr uint64_t IPC_MAGIC = 0x4350493030324247ull;  // "GB200IPC"
-constexpr int IPC_ARRAYS = 12;
+constexpr int IPC_ARRAYS = 14;
 
 struct IpcArray { uint64_t bytes; cudaIpcMemHandle_t handle; };
 
@@ -1188,6 +1318,7 @@ struct IpcHeader {
     WindowPlan window;
     uint64_t ckpt_ok, ckpt_shift, ckpt_entries, ckpt_bytes, ckpt_build_us, ckpt_max_segments;
     uint64_t has_graph, graph_sequences, graph_bytes;
+    uint64_t locate_ok, locate_shift, locate_samples, locate_bytes, locate_build_us;
     uint64_t source_device;
     IpcArray arrays[IPC_ARRAYS];
 };
@@ -1233,13 +1364,16 @@ struct BlobReader {
 void ipc_arrays(const gbwt_b200_index* ix, void* ptrs[IPC_ARRAYS], uint64_t sizes[IPC_ARRAYS]) {
     const uint64_t seq_bytes = std::max<uint64_t>(256, ix->sequences * sizeof(uint64_t));
     void* p[IPC_ARRAYS] = {ix->d_desc, ix->d_bodies, ix->d_edges, ix->d_endmarker, ix->d_skips, ix->d_stage_body, ix->d_seq_len,
-                           ix->d_dna_len, ix->d_ckpt_table, ix->d_ckpt_first, ix->d_label_starts, ix->d_label_bytes};
+                           ix->d_dna_len, ix->d_ckpt_table, ix->d_ckpt_first, ix->d_label_starts, ix->d_label_bytes,
+                           ix->d_locate_first, ix->d_locate_samples};
     const uint64_t b[IPC_ARRAYS] = {ix->bytes[0], ix->bytes[1], ix->bytes[2], ix->bytes[3],
                                     (ix->view.records + 1) * 16, (ix->view.records / STAGE_GRANULE + 2) * sizeof(uint32_t), 4 * seq_bytes, seq_bytes,
                                     ix->ckpt_ok ? ix->ckpt_entries * sizeof(Checkpoint) : 0,
                                     ix->ckpt_ok ? (ix->view.sequences + 1) * sizeof(uint32_t) : 0,
                                     ix->has_graph ? (ix->graph.sequences + 1) * 8 : 0,
-                                    ix->has_graph ? ix->graph_bytes - (ix->graph.sequences + 1) * 8 : 0};
+                                    ix->has_graph ? ix->graph_bytes - (ix->graph.sequences + 1) * 8 : 0,
+                                    ix->locate_ok ? (ix->view.records + 1) * sizeof(uint32_t) : 0,
+                                    ix->locate_ok ? ix->locate_samples * sizeof(LocateSample) : 0};
     for (int i = 0; i < IPC_ARRAYS; i++) { ptrs[i] = p[i]; sizes[i] = p[i] != nullptr ? b[i] : 0; }
 }
 
@@ -1254,7 +1388,7 @@ int gbwt_b200_index_export_ipc(const gbwt_b200_index* ix, void** blob, size_t* l
     CUDA_TRY(cudaDeviceSynchronize());  // everything the build enqueued has landed
     IpcHeader h;
     std::memset(&h, 0, sizeof(h));
-    h.magic = IPC_MAGIC; h.version = 1;
+    h.magic = IPC_MAGIC; h.version = 2;
     h.sequences = ix->sequences; h.size = ix->size; h.offset = ix->offset; h.alphabet_size = ix->alphabet_size; h.flags = ix->flags;
     h.records = ix->view.records; h.endmarker_len = ix->view.endmarker_len; h.bidirectional = ix->view.bidirectional;
     h.edges_valid = ix->view.edges_valid; h.walk_limit = ix->view.walk_limit;
@@ -1267,6 +1401,8 @@ int gbwt_b200_index_export_ipc(const gbwt_b200_index* ix, void** blob, size_t* l
     h.ckpt_ok = ix->ckpt_ok; h.ckpt_shift = ix->ckpt_shift; h.ckpt_entries = ix->ckpt_entries; h.ckpt_bytes = ix->ckpt_bytes;
     h.ckpt_build_us = ix->ckpt_build_us; h.ckpt_max_segments = ix->ckpt.max_segments;
     h.has_graph = ix->has_graph; h.graph_sequences = ix->graph.sequences; h.graph_bytes = ix->graph_bytes;
+    h.locate_ok = ix->locate_ok; h.locate_shift = ix->locate_shift; h.locate_samples = ix->locate_samples;
+    h.locate_bytes = ix->locate_bytes; h.locate_build_us = ix->locate_build_us;
     h.source_device = static_cast<uint64_t>(ix->device);
     void* ptrs[IPC_ARRAYS];
     uint64_t sizes[IPC_ARRAYS];
@@ -1295,7 +1431,7 @@ int gbwt_b200_index_import_ipc(const void* blob, size_t len, int device, gbwt_b2
     if (len < sizeof(IpcHeader)) return fail(GBWT_B200_E_INVALID_DATA, "not an exported index");
     IpcHeader h;
     std::memcpy(&h, blob, sizeof(h));
-    if (h.magic != IPC_MAGIC || h.version != 1) return fail(GBWT_B200_E_INVALID_DATA, "not an exported index");
+    if (h.magic != IPC_MAGIC || h.version != 2) return fail(GBWT_B200_E_INVALID_DATA, "not an exported index");
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
         cudaGetLastError();
@@ -1321,7 +1457,8 @@ int gbwt_b200_index_import_ipc(const void* blob, size_t len, int device, gbwt_b2
         if (!rd.ok) { delete ix; return fail(GBWT_B200_E_INVALID_DATA, "truncated exported index"); }
         // the arrays: open the exporter's allocation, copy it device to device, close it
         void** slots[IPC_ARRAYS] = {&ix->d_desc, &ix->d_bodies, &ix->d_edges, &ix->d_endmarker, &ix->d_skips, &ix->d_stage_body, &ix->d_seq_len,
-                                    &ix->d_dna_len, &ix->d_ckpt_table, &ix->d_ckpt_first, &ix->d_label_starts, &ix->d_label_bytes};
+                                    &ix->d_dna_len, &ix->d_ckpt_table, &ix->d_ckpt_first, &ix->d_label_starts, &ix->d_label_bytes,
+                                    &ix->d_locate_first, &ix->d_locate_samples};
         int rc = GBWT_B200_OK;
         for (int i = 0; i < IPC_ARRAYS && rc == GBWT_B200_OK; i++) {
             if (h.arrays[i].bytes == 0) continue;
@@ -1374,6 +1511,16 @@ int gbwt_b200_index_import_ipc(const void* blob, size_t len, int device, gbwt_b2
             ix->graph_bytes = h.graph_bytes;
             ix->has_graph = true;
         }
+        if (h.locate_ok) {
+            // (an index without samples has a zero-sized sample array: the table comes over only with its `first`)
+            ix->locate_ok = ix->d_locate_first != nullptr;
+            if (ix->locate_ok && ix->d_locate_samples == nullptr && cudaMalloc(&ix->d_locate_samples, 256) != cudaSuccess) {
+                gbwt_b200_index_destroy(ix);
+                return cuda_fail(cudaGetLastError(), "cudaMalloc(locate table)");
+            }
+            ix->locate_shift = static_cast<uint32_t>(h.locate_shift); ix->locate_samples = h.locate_samples;
+            ix->locate_bytes = h.locate_bytes; ix->locate_build_us = h.locate_build_us;
+        }
         build_dna_checkpoints(ix);  // (a table of the importer's own: a short count pass, not worth a handle in the blob)
         *out = ix;
         return GBWT_B200_OK;
@@ -1393,7 +1540,7 @@ void gbwt_b200_index_destroy(gbwt_b200_index* ix) {
     {
         DeviceScope scope(ix->device);
         cudaFree(ix->d_desc); cudaFree(ix->d_bodies); cudaFree(ix->d_edges); cudaFree(ix->d_endmarker); cudaFree(ix->d_skips); cudaFree(ix->d_stage_body); cudaFree(ix->d_ckpt_table); cudaFree(ix->d_ckpt_first); cudaFree(ix->d_seq_len); cudaFree(ix->d_dna_len); cudaFree(ix->d_ckpt_dna);
-        cudaFree(ix->d_label_starts); cudaFree(ix->d_label_bytes);
+        cudaFree(ix->d_label_starts); cudaFree(ix->d_label_bytes); cudaFree(ix->d_locate_first); cudaFree(ix->d_locate_samples);
     }
     delete ix;
 }
@@ -1420,6 +1567,13 @@ uint64_t gbwt_b200_dense4_records(const gbwt_b200_index* ix) { return ix ? ix->f
 void gbwt_b200_checkpoint_info(const gbwt_b200_index* ix, uint64_t info[6]) {
     if (ix == nullptr || info == nullptr) return;
     const uint64_t values[6] = {ix->ckpt_ok, uint64_t(1) << ix->ckpt_shift, ix->ckpt_entries, ix->ckpt_bytes, ix->ckpt_build_us, ix->ckpt.max_segments};
+    for (int i = 0; i < 6; i++) info[i] = values[i];
+}
+
+void gbwt_b200_locate_info(const gbwt_b200_index* ix, uint64_t info[6]) {
+    if (ix == nullptr || info == nullptr) return;
+    const uint64_t values[6] = {ix->locate_ok, ix->locate_ok ? uint64_t(1) << ix->locate_shift : 0, ix->locate_samples, ix->locate_bytes,
+                                ix->locate_build_us, ix->locate_steps.load()};
     for (int i = 0; i < 6; i++) info[i] = values[i];
 }
 
@@ -1453,7 +1607,8 @@ uint64_t gbwt_b200_device_bytes(const gbwt_b200_index* ix, uint64_t breakdown[10
         for (int i = 0; i < 6; i++) breakdown[4 + i] = ix->format_counts[i];
         breakdown[4 + FMT_DENSE2] += ix->format_counts[FMT_DENSE4];  // both dense formats in one slot (gbwt_b200_dense4_records tells them apart)
     }
-    return ix->bytes[0] + ix->bytes[1] + ix->bytes[2] + ix->bytes[3] + ix->skip_bytes + ix->graph_bytes + ix->ckpt_bytes;
+    return ix->bytes[0] + ix->bytes[1] + ix->bytes[2] + ix->bytes[3] + ix->skip_bytes + ix->graph_bytes + ix->ckpt_bytes +
+           (ix->locate_ok ? ix->locate_bytes : 0);
 }
 
 // ---- device-pointer entry points ---------------------------------------------------------------------
@@ -1525,6 +1680,29 @@ int gbwt_b200_extract_device(const gbwt_b200_index* ix, const uint64_t* d_seq_id
     DEVICE_ENTRY_PROLOGUE(ix);
     if (d_nodes == nullptr || d_out_offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null output");
     return launch_extract(ix, d_seq_ids, m, d_out_offsets, 0, d_nodes, d_lengths, static_cast<cudaStream_t>(stream));
+}
+
+int gbwt_b200_locate_device(const gbwt_b200_index* ix, const gbwt_b200_pos* d_positions, size_t n, gbwt_b200_occurrence* d_out, void* stream) {
+    DEVICE_ENTRY_PROLOGUE(ix);
+    if (int rc = check_samples(ix)) return rc;
+    if (n > 0 && (d_positions == nullptr || d_out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    return launch_locate_positions(ix, d_positions, n, d_out, static_cast<cudaStream_t>(stream));
+}
+int gbwt_b200_locate_states_device(const gbwt_b200_index* ix, const gbwt_b200_state* d_states, size_t n, const uint64_t* d_out_offsets,
+                                   gbwt_b200_occurrence* d_out, uint64_t* d_counts, void* stream) {
+    DEVICE_ENTRY_PROLOGUE(ix);
+    if (int rc = check_samples(ix)) return rc;
+    if (n > 0 && (d_states == nullptr || (d_out != nullptr && d_out_offsets == nullptr) || (d_out == nullptr && d_counts == nullptr)))
+        return fail(GBWT_B200_E_ARGUMENT, "null array");
+    // (the scan of a chunk is indexed with 64-bit CUB offsets; chunks keep each launch's temporary arrays bounded)
+    const size_t chunk = size_t(1) << 30;
+    for (size_t begin = 0; begin < n; begin += chunk) {
+        const size_t count = std::min(chunk, n - begin);
+        int rc = launch_locate_state_batch(ix, d_states + begin, count, d_out_offsets != nullptr ? d_out_offsets + begin : nullptr, 0, d_out,
+                                           d_counts != nullptr ? d_counts + begin : nullptr, static_cast<cudaStream_t>(stream));
+        if (rc != GBWT_B200_OK) return rc;
+    }
+    return GBWT_B200_OK;
 }
 
 int gbwt_b200_dna_lengths_device(const gbwt_b200_index* ix, const uint64_t* d_seq_ids, size_t m, uint64_t* d_lengths, void* stream) {
@@ -1758,6 +1936,77 @@ int gbwt_b200_extract_dna(const gbwt_b200_index* ix, const uint64_t* seq_ids, si
                              [&](const uint64_t* d_ids, size_t count, const uint64_t* d_offsets, uint64_t base, void* d_out, uint64_t* d_lengths, cudaStream_t s) {
                                  return launch_extract_dna(ix, d_ids, count, d_offsets, base, endmarker, static_cast<uint8_t*>(d_out), d_lengths, s);
                              });
+}
+
+int gbwt_b200_locate(const gbwt_b200_index* ix, const gbwt_b200_pos* positions, size_t n, gbwt_b200_occurrence* out) {
+    if (int rc = check_index(ix)) return rc;
+    if (int rc = check_samples(ix)) return rc;
+    if (n > 0 && (positions == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    std::vector<HostArray> arrays = {{positions, nullptr, sizeof(gbwt_b200_pos)}, {nullptr, out, sizeof(gbwt_b200_occurrence)}};
+    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_pos)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_locate_positions(ix, static_cast<gbwt_b200_pos*>(d[0]), count, static_cast<gbwt_b200_occurrence*>(d[1]), s);
+    });
+}
+
+// Chunks of states whose output slots hold at most 16 Mi occurrences (at least one state), like gbwt_b200_follow.
+int gbwt_b200_locate_states(const gbwt_b200_index* ix, const gbwt_b200_state* states, size_t n, const uint64_t* out_offsets,
+                            gbwt_b200_occurrence* out, uint64_t* counts) {
+    if (int rc = check_index(ix)) return rc;
+    if (int rc = check_samples(ix)) return rc;
+    if (n == 0) return GBWT_B200_OK;
+    if (states == nullptr || (out != nullptr && out_offsets == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    if (out == nullptr) {
+        if (counts == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null array");
+        std::vector<HostArray> arrays = {{states, nullptr, sizeof(gbwt_b200_state)}, {nullptr, counts, 8}};
+        return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_state)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+            return launch_locate_state_batch(ix, static_cast<gbwt_b200_state*>(d[0]), count, nullptr, 0, nullptr, static_cast<uint64_t*>(d[1]), s);
+        });
+    }
+    if (!offsets_valid(out_offsets, n)) return fail(GBWT_B200_E_ARGUMENT, "out_offsets must be non-decreasing");
+    DeviceScope scope(ix->device);
+    if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
+    cudaStream_t s;
+    CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    int rc = GBWT_B200_OK;
+    for (size_t i0 = 0; i0 < n && rc == GBWT_B200_OK;) {
+        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, size_t(1) << 22, uint64_t(16) << 20);
+        const size_t count = i1 - i0;
+        const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
+        gbwt_b200_state* d_states = nullptr;
+        gbwt_b200_occurrence* d_out = nullptr;
+        uint64_t *d_offsets = nullptr, *d_counts = nullptr;
+        auto alloc = [&](void** p, size_t bytes) {
+            cudaError_t e = cudaMallocAsync(p, std::max<size_t>(16, bytes), s);
+            if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaMallocAsync");
+        };
+        alloc(reinterpret_cast<void**>(&d_states), count * sizeof(gbwt_b200_state));
+        alloc(reinterpret_cast<void**>(&d_out), cap * sizeof(gbwt_b200_occurrence));
+        alloc(reinterpret_cast<void**>(&d_offsets), (count + 1) * 8);
+        alloc(reinterpret_cast<void**>(&d_counts), count * 8);
+        if (rc == GBWT_B200_OK) {
+            // slots may be larger than the answers: the slack must not carry stale pool memory back to the caller
+            cudaError_t e = cap > 0 ? cudaMemsetAsync(d_out, 0xFF, cap * sizeof(gbwt_b200_occurrence), s) : cudaSuccess;
+            if (e == cudaSuccess) e = cudaMemcpyAsync(d_states, states + i0, count * sizeof(gbwt_b200_state), cudaMemcpyHostToDevice, s);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(d_offsets, out_offsets + i0, (count + 1) * 8, cudaMemcpyHostToDevice, s);
+            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
+        }
+        if (rc == GBWT_B200_OK) rc = launch_locate_state_batch(ix, d_states, count, d_offsets, base, d_out, d_counts, s);
+        if (rc == GBWT_B200_OK) {
+            cudaError_t e = cudaSuccess;
+            if (cap > 0) e = cudaMemcpyAsync(out + base, d_out, cap * sizeof(gbwt_b200_occurrence), cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess && counts != nullptr) e = cudaMemcpyAsync(counts + i0, d_counts, count * 8, cudaMemcpyDeviceToHost, s);
+            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
+        }
+        if (d_states) cudaFreeAsync(d_states, s);
+        if (d_out) cudaFreeAsync(d_out, s);
+        if (d_offsets) cudaFreeAsync(d_offsets, s);
+        if (d_counts) cudaFreeAsync(d_counts, s);
+        i0 = i1;
+    }
+    cudaError_t e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
+    cudaStreamDestroy(s);
+    return rc;
 }
 
 int gbwt_b200_node_sequence_lengths(const gbwt_b200_index* ix, const uint64_t* node_ids, size_t n, uint64_t* lengths) {

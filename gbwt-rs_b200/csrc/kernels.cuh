@@ -9,6 +9,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "find_lean.cuh"
 #include "record_scan.cuh"
 
@@ -757,6 +759,10 @@ __device__ __forceinline__ bool walk_bubble_step(Desc& cur_d, Quad& cur_k, Desc&
 // CHECKED = false relies on IndexView::edges_valid (no bounds tests on edge targets).
 // `limit`: stop once at least that many nodes have been handed to the sink (checked when the lanes are flushed, so
 // the walk may run up to 32 nodes further; the sink clips).
+// A sink that also wants the position of the sequence's last node defines last_node(node, offset, index) (LocateSink).
+template <class Sink, class = void> struct sink_wants_last_node : std::false_type {};
+template <class Sink> struct sink_wants_last_node<Sink, std::void_t<decltype(&Sink::last_node)>> : std::true_type {};
+
 template <bool CHECKED, class Sink>
 __device__ __forceinline__ uint64_t walk_sequence_warp(const IndexView& ix, uint64_t id, Sink& sink, uint32_t ahead,
                                                        uint64_t limit = ~0ull) {
@@ -889,6 +895,8 @@ __device__ __forceinline__ uint64_t walk_sequence_warp(const IndexView& ix, uint
         else { d = t1; k = s1; }
     }
     if (in_group != 0) sink.group(static_cast<uint64_t>(mine), in_group, flushed);
+    // (node, offset) is the position of the last node the walk emitted, unless it stopped at a flush (walk_limit)
+    if constexpr (sink_wants_last_node<Sink>::value) { if (in_group != 0) sink.last_node(node, offset, flushed + in_group - 1); }
     sink.finish();
     return flushed + in_group;
 }
@@ -1341,6 +1349,84 @@ __global__ void __launch_bounds__(BLOCK_THREADS) k_checkpoint_scatter(const Pool
     }
 }
 
+
+// ---- locate samples (gbwt_b200_locate; DESIGN.md "Locate") ---------------------------------------------------------
+// The same walk as the checkpoints, with the table inverted: indexed by BWT position instead of by sequence. Every
+// sample is emitted as a sort key (record << 32 | offset) and the sample itself; locate.cu sorts them into the table.
+// Rule: a sample at the first flush at or after every multiple of 2^shift (flushes are at most 32 nodes apart), and at
+// the sequence's last node. A locate walk therefore meets one within 2^shift + 32 LF steps. The last node is sampled
+// because that is where every walk would otherwise leave the sequence: GBWT::forward is None there, and nothing in the
+// format ties the endmarker position it would enter to the sequence id.
+struct LocateSink {
+    static constexpr bool CHECKPOINTS = true;
+    uint64_t* keys;
+    LocateSample* samples;
+    unsigned long long* used;
+    uint64_t cap, base, records;  // base = alphabet offset (record = node - base)
+    uint32_t seq, shift;
+    uint64_t next, last;  // first index that wants a sample; index of the last sample emitted (~0 = none)
+    __device__ __forceinline__ void emit(uint32_t node, uint32_t offset, uint64_t index) {
+        last = index;
+        // (a damaged index can lead a walk to a node without a record: no position there can be located)
+        if ((threadIdx.x & 31u) != 0 || node <= base || node - base >= records) return;
+        const unsigned long long slot = atomicAdd(used, 1ull);
+        if (slot >= cap) return;  // (the caller sees used > cap and fails: cannot happen on a consistent index)
+        keys[slot] = (static_cast<uint64_t>(node - base) << 32) | offset;
+        LocateSample e;
+        e.offset = offset; e.seq = seq; e.index = index;
+        samples[slot] = e;
+    }
+    __device__ __forceinline__ void group(uint64_t, uint32_t, uint64_t) {}
+    __device__ __forceinline__ void finish() {}
+    __device__ __forceinline__ void checkpoint(uint32_t node, uint32_t offset, uint64_t index) {
+        if (index < next) return;
+        next = ((index >> shift) + 1) << shift;
+        emit(node, offset, index);
+    }
+    __device__ __forceinline__ void last_node(uint32_t node, uint32_t offset, uint64_t index) {
+        if (index != last) emit(node, offset, index);
+    }
+};
+
+// One warp per sequence (shift >= 5: the flushes are denser than the samples).
+template <bool CHECKED>
+__global__ void __launch_bounds__(128) k_build_locate(IndexView ix, uint32_t shift, uint64_t* __restrict__ keys,
+                                                       LocateSample* __restrict__ samples, unsigned long long* __restrict__ used,
+                                                       uint64_t cap, uint32_t ahead) {
+    const size_t warp = (static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x) / 32;
+    const size_t warps = (static_cast<size_t>(gridDim.x) * blockDim.x) / 32;
+    for (size_t id = warp; id < ix.sequences; id += warps) {
+        LocateSink sink{keys, samples, used, cap, ix.offset, ix.records, static_cast<uint32_t>(id), shift, 0, ~0ull};
+        walk_sequence_warp<CHECKED>(ix, id, sink, ahead);
+    }
+}
+
+// Intervals shorter than a flush (shift < 5; shift 0 is the whole document array, for tests): one lane per sequence
+// walks it with GBWT::forward and samples exactly every multiple of 2^shift and the last node.
+__global__ void __launch_bounds__(BLOCK_THREADS) k_build_locate_lanes(IndexView ix, uint32_t shift, uint64_t* __restrict__ keys,
+                                                                       LocateSample* __restrict__ samples,
+                                                                       unsigned long long* __restrict__ used, uint64_t cap) {
+    GBWT_GRID_STRIDE(id, ix.sequences) {
+        gbwt_b200_pos pos;
+        if (!gbwt_start(ix, id, pos)) continue;
+        for (uint64_t j = 0; j <= ix.walk_limit; j++) {
+            gbwt_b200_pos next;
+            const bool more = gbwt_forward(ix, pos, next);
+            const bool located = pos.node > ix.offset && pos.node - ix.offset < ix.records;  // (see LocateSink::emit)
+            if (located && (!more || (j & ((uint64_t(1) << shift) - 1)) == 0)) {
+                const unsigned long long slot = atomicAdd(used, 1ull);
+                if (slot < cap) {
+                    keys[slot] = ((pos.node - ix.offset) << 32) | pos.offset;
+                    LocateSample e;
+                    e.offset = static_cast<uint32_t>(pos.offset); e.seq = static_cast<uint32_t>(id); e.index = j;
+                    samples[slot] = e;
+                }
+            }
+            if (!more) break;
+            pos = next;
+        }
+    }
+}
 
 // Work item (segment j, block of 32 batch entries): lane l walks segment j of sequence ids[32 * block + l] from its
 // checkpoint to the next one (or to the end of the sequence): Record::lf (src/bwt.rs:480-496) per step, two nodes per

@@ -128,6 +128,16 @@ struct CheckpointView {
     uint32_t lookahead;        // records ahead of the walks at which a warp touches the index once per round (0 = off)
 };
 
+// Locate samples (kernels.cuh: k_build_locate, locate.cu): (sequence, index) at some positions of every sequence, indexed
+// by BWT position. The samples of record r are samples[first[r] .. first[r + 1]), sorted by offset.
+struct LocateSample { uint32_t offset, seq; uint64_t index; };  // position (record, offset) is node `index` of sequence `seq`
+static_assert(sizeof(LocateSample) == 16, "samples are loaded with one vector load");
+struct LocateView {
+    const uint32_t* first;          // [records + 1]
+    const LocateSample* samples;
+    uint64_t max_steps;             // LF steps after which a walk gives up (none): the sample bound plus slack
+};
+
 // Magic multiplier for q = b / sigma, 0 <= b < 256, 1 <= sigma <= 256: q = (b * magic) >> 16.
 GBWT_HD uint32_t div_magic(uint32_t sigma) { return 65536u / sigma + 1u; }
 

@@ -661,13 +661,9 @@ GBWT_HD bool gbwt_extend_backward(const IndexView& ix, const gbwt_b200_bdstate& 
     return true;
 }
 
-// GBWT::forward + Record::lf, src/gbwt.rs:222-229, src/bwt.rs:480-496. False = None.
-GBWT_HD bool gbwt_forward(const IndexView& ix, const gbwt_b200_pos& pos, gbwt_b200_pos& out) {
-    const uint64_t node = pos.node, offset = pos.offset;
+// Record::lf at `offset` of the record whose descriptor is `d` (src/bwt.rs:480-496). False = None.
+GBWT_HD bool lf_in_record(const IndexView& ix, const Desc& d, uint64_t offset, gbwt_b200_pos& out) {
     set_none(out);
-    uint64_t rec;
-    if (node < ix.offset + 1 || !record_of(ix, node, rec)) return false;
-    const Desc d = load_desc(ix, rec);
     const uint32_t fmt = d.fmt();
     if (fmt == FMT_EMPTY || offset >= d.total_len()) return false;
     const uint32_t i = static_cast<uint32_t>(offset);
@@ -691,6 +687,14 @@ GBWT_HD bool gbwt_forward(const IndexView& ix, const gbwt_b200_pos& pos, gbwt_b2
     if (e.node == 0) return false;  // successor is the endmarker: the sequence ends (src/bwt.rs:485-486)
     out.node = e.node; out.offset = static_cast<uint64_t>(e.offset) + rank_i;
     return true;
+}
+
+// GBWT::forward + Record::lf, src/gbwt.rs:222-229, src/bwt.rs:480-496. False = None.
+GBWT_HD bool gbwt_forward(const IndexView& ix, const gbwt_b200_pos& pos, gbwt_b200_pos& out) {
+    set_none(out);
+    uint64_t rec;
+    if (pos.node < ix.offset + 1 || !record_of(ix, pos.node, rec)) return false;
+    return lf_in_record(ix, load_desc(ix, rec), pos.offset, out);
 }
 
 // GBWT::start, src/gbwt.rs:213-219.
@@ -1094,6 +1098,50 @@ GBWT_HD uint64_t walk_sequence(const IndexView& ix, uint64_t id, uint64_t* out, 
         pos = next;
     }
     return n;
+}
+
+// locate(node, offset) (gbwt_b200.h; the C++ GBWT's locate(node, i) is the model): the walk Record::lf takes from the
+// position until it meets a locate sample; the answer is the sample's sequence and its index minus the steps taken.
+// Per step the record's sample range and its descriptor are requested together: most records hold no sample, and the
+// descriptor is what the LF step needs next. The walk never uses the two-hop shortcuts (IndexView::skips): they step over
+// the middle node, and a sample there would be missed. False (and {UINT64_MAX, UINT64_MAX}) where the position does not
+// exist, and where no sample is met within lv.max_steps steps (a damaged index: a consistent one always meets one).
+// `steps` receives the number of LF steps taken.
+GBWT_HD bool gbwt_locate(const IndexView& ix, const LocateView& lv, uint64_t node, uint64_t offset, gbwt_b200_occurrence& out,
+                         uint64_t& steps) {
+    out.sequence = ~0ull; out.index = ~0ull;
+    steps = 0;
+    uint64_t rec;
+    // (offsets are 32-bit in the layout: a larger one must not be truncated onto a sampled offset)
+    if (node < ix.offset + 1 || !record_of(ix, node, rec) || offset > 0xFFFFFFFFull) return false;
+    gbwt_b200_pos pos;
+    pos.node = node; pos.offset = offset;
+    for (uint64_t s = 0;; s++) {
+        const uint32_t lo = GBWT_LDG(lv.first + rec), hi = GBWT_LDG(lv.first + rec + 1);
+        const Desc d = load_desc(ix, rec);
+        if (lo < hi) {
+            // samples of a record are sorted by offset: the last one at or below this offset
+            const uint32_t i = static_cast<uint32_t>(pos.offset);
+            uint32_t a = lo, b = hi;
+            while (b - a > 1) {
+                const uint32_t mid = a + (b - a) / 2;
+                if (GBWT_LDG(&lv.samples[mid].offset) <= i) a = mid; else b = mid;
+            }
+            if (GBWT_LDG(&lv.samples[a].offset) == i) {
+                const uint64_t index = GBWT_LDG(&lv.samples[a].index);
+                steps = s;
+                if (index < s) return false;  // (a damaged index)
+                out.sequence = GBWT_LDG(&lv.samples[a].seq);
+                out.index = index - s;
+                return true;
+            }
+        }
+        if (s >= lv.max_steps) { steps = s; return false; }
+        gbwt_b200_pos next;
+        // (also the validity test of the first position: no record, an empty one, or an offset past its end -> None)
+        if (!lf_in_record(ix, d, pos.offset, next) || !record_of(ix, next.node, rec) || next.node < ix.offset + 1) { steps = s; return false; }
+        pos = next;
+    }
 }
 
 }  // namespace gbwt_b200

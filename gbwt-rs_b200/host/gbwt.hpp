@@ -133,6 +133,28 @@ public:
         return std::vector<std::size_t>(paths.second.begin(), paths.second.end());
     }
 
+    // locate (beyond the crate; the C++ GBWT's locate is the model, include/gbwt_b200.h): (sequence, index) of a position,
+    // nullopt where there is no such position; the occurrences of a state in offset order. Needs an index created with
+    // GBWT_B200_LAYOUT_LOCATE (throws otherwise).
+    std::optional<std::pair<std::size_t, std::size_t>> locate(Pos pos) const {
+        gbwt_b200_pos in{pos.node, pos.offset};
+        gbwt_b200_occurrence out;
+        check(gbwt_b200_locate(h_, &in, 1, &out));
+        if (out.sequence == UINT64_MAX) return std::nullopt;
+        return std::make_pair(static_cast<std::size_t>(out.sequence), static_cast<std::size_t>(out.index));
+    }
+    std::vector<std::pair<std::size_t, std::size_t>> locate(const SearchState& state) const {
+        const gbwt_b200_state in = from_state(state);
+        const uint64_t n = state.range.second > state.range.first ? state.range.second - state.range.first : 0;
+        const uint64_t offsets[2] = {0, n};
+        std::vector<gbwt_b200_occurrence> raw(n);
+        uint64_t count = 0;
+        check(gbwt_b200_locate_states(h_, &in, 1, offsets, raw.data(), &count));
+        std::vector<std::pair<std::size_t, std::size_t>> out;
+        for (const auto& o : raw) out.emplace_back(static_cast<std::size_t>(o.sequence), static_cast<std::size_t>(o.index));
+        return out;
+    }
+
     // Subpath search, src/gbwt.rs:269-304.
     std::optional<SearchState> find(std::size_t node) const {
         uint64_t in = node;

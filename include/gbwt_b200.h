@@ -56,7 +56,8 @@ enum {
     GBWT_B200_E_CUDA = 5,              /* CUDA runtime error; see gbwt_b200_last_error() */
     GBWT_B200_E_ARGUMENT = 6,          /* NULL handle / pointer, bad layout policy, ... */
     GBWT_B200_E_NO_DEVICE = 7,         /* no CUDA device: there is deliberately no CPU fallback */
-    GBWT_B200_E_NO_GRAPH = 8           /* node sequences requested from an index that has no graph (not a GBZ) */
+    GBWT_B200_E_NO_GRAPH = 8,          /* node sequences requested from an index that has no graph (not a GBZ) */
+    GBWT_B200_E_NO_SAMPLES = 9         /* locate on an index created without GBWT_B200_LAYOUT_LOCATE */
 };
 
 /* ---- value types ------------------------------------------------------------------------------ */
@@ -66,6 +67,9 @@ typedef struct { uint64_t node, offset; } gbwt_b200_pos;
 typedef struct { uint64_t node, start, end; } gbwt_b200_state;
 /* BidirectionalState, src/gbwt.rs:484-528. */
 typedef struct { gbwt_b200_state forward, reverse; } gbwt_b200_bdstate;
+/* What locate answers for one BWT position: node number `index` (from 0) of GBWT::sequence(`sequence`). {UINT64_MAX,
+ * UINT64_MAX} where there is no such position. */
+typedef struct { uint64_t sequence, index; } gbwt_b200_occurrence;
 
 typedef struct gbwt_b200_index gbwt_b200_index;
 
@@ -78,7 +82,11 @@ enum {
      * independent segments instead of one dependent chain per sequence (results identical; see DESIGN.md).
      * Built by default for indexes of 4 Mi path nodes or more. */
     GBWT_B200_LAYOUT_CHECKPOINTS = 0x100,    /* build them whatever the size */
-    GBWT_B200_LAYOUT_NO_CHECKPOINTS = 0x200  /* never build them (extraction walks whole chains) */
+    GBWT_B200_LAYOUT_NO_CHECKPOINTS = 0x200, /* never build them (extraction walks whole chains) */
+    /* Locate samples (opt-in): while the index is created, one walk over every sequence samples its positions, so that
+     * gbwt_b200_locate can turn a BWT position into (sequence, index). Without this flag no locate entry point works
+     * (GBWT_B200_E_NO_SAMPLES) and nothing else changes. See "locate" below and DESIGN.md. */
+    GBWT_B200_LAYOUT_LOCATE = 0x400
 };
 
 /* ---- construction (replaces GBWT::load / serialize::load_from, src/gbwt.rs:402-438; the embedded
@@ -161,6 +169,11 @@ GBWT_B200_API void gbwt_b200_checkpoint_info(const gbwt_b200_index* index, uint6
  * [12] device time of the window kernel launches in nanoseconds, [13] number of those launches. */
 GBWT_B200_API void gbwt_b200_window_info(const gbwt_b200_index* index, uint64_t info[14]);
 
+/* Locate samples of this index: [0] present, [1] interval (positions of a sequence), [2] samples, [3] bytes of HBM, [4]
+ * microseconds the build took on the device, and -- only counted when GBWT_B200_LOCATE_STATS=1 -- [5] LF steps taken by
+ * locate walks. */
+GBWT_B200_API void gbwt_b200_locate_info(const gbwt_b200_index* index, uint64_t info[6]);
+
 /* ---- unidirectional search -------------------------------------------------------------------- */
 /* GBWT::find (src/gbwt.rs:269-281) for n nodes. */
 GBWT_B200_API int gbwt_b200_find(const gbwt_b200_index* index, const uint64_t* nodes, size_t n, gbwt_b200_state* out);
@@ -226,6 +239,27 @@ GBWT_B200_API int gbwt_b200_sequence_lengths(const gbwt_b200_index* index, const
 GBWT_B200_API int gbwt_b200_extract(const gbwt_b200_index* index, const uint64_t* seq_ids, size_t m,
                                    const uint64_t* out_offsets, uint64_t* nodes, uint64_t* lengths);
 
+/* ---- locate: which sequences, and where on them (beyond the reference crate) -------------------------------------
+ * The reference crate has no locate: it carries the document-array samples of a GBWT file as opaque bytes
+ * (src/gbwt.rs:100, 417). The model is the C++ GBWT's `locate(node, i)` and `locate(state)` (gbwt/gbwt.h, backed by
+ * its DASamples). The answer is defined by what the crate does provide: position (node, i) with node >= first_node()
+ * and i < Record::len() lies on exactly one sequence s, as node number j (from 0) of GBWT::sequence(s) -- the j-th
+ * position that GBWT::start(s) and j GBWT::forward steps reach (src/gbwt.rs:213-229, 253-261, 557-568). locate(node, i)
+ * = {s, j}. {UINT64_MAX, UINT64_MAX} where no such position exists: node == ENDMARKER or below first_node(), a node
+ * without a record or with an empty record, i >= len, and, on a damaged index, a walk that meets no sample within its
+ * bound. Requires an index created with GBWT_B200_LAYOUT_LOCATE (GBWT_B200_E_NO_SAMPLES otherwise).
+ * How: the samples hold (sequence, index) at every 2^shift-th node of every sequence (GBWT_B200_LOCATE_SHIFT, default
+ * 10) and at its last node; a position walks forward with Record::lf until it meets one, then subtracts its steps. */
+GBWT_B200_API int gbwt_b200_locate(const gbwt_b200_index* index, const gbwt_b200_pos* positions, size_t n,
+                                  gbwt_b200_occurrence* out);
+/* The occurrences of a SearchState {node, start, end}: locate of (node, start) .. (node, end - 1), in offset order,
+ * end - start of them, none for a None state. counts[i] = end - start (0 for None), so a caller can size the output
+ * without a first call; the occurrences of state i are written to out[out_offsets[i] ..], at most
+ * out_offsets[i+1] - out_offsets[i] of them (what is left of a longer slot is unspecified). out may be NULL (counts
+ * only). The C++ GBWT's locate(state) is the sorted, deduplicated set of the .sequence fields of this answer. */
+GBWT_B200_API int gbwt_b200_locate_states(const gbwt_b200_index* index, const gbwt_b200_state* states, size_t n,
+                                         const uint64_t* out_offsets, gbwt_b200_occurrence* out, uint64_t* counts);
+
 /* ---- node sequences (GBZ files only; GBWT_B200_E_NO_GRAPH otherwise) ------------------------------ */
 /* GBZ::sequence_len / GBZ::sequence (src/gbz.rs:292-306) for n original-graph node identifiers: lengths[i] is the
  * label length, UINT64_MAX where the reference returns None (GBZ::has_node is false, src/gbz.rs:286-289). */
@@ -275,6 +309,12 @@ GBWT_B200_API int gbwt_b200_sequence_lengths_device(const gbwt_b200_index* index
 GBWT_B200_API int gbwt_b200_extract_device(const gbwt_b200_index* index, const uint64_t* d_seq_ids, size_t m,
                                           const uint64_t* d_out_offsets, uint64_t* d_nodes, uint64_t* d_lengths,
                                           void* stream);
+
+GBWT_B200_API int gbwt_b200_locate_device(const gbwt_b200_index* index, const gbwt_b200_pos* d_positions, size_t n,
+                                         gbwt_b200_occurrence* d_out, void* stream);
+GBWT_B200_API int gbwt_b200_locate_states_device(const gbwt_b200_index* index, const gbwt_b200_state* d_states, size_t n,
+                                                const uint64_t* d_out_offsets, gbwt_b200_occurrence* d_out,
+                                                uint64_t* d_counts, void* stream);
 
 /* ---- utilities -------------------------------------------------------------------------------- */
 /* Page-locked host buffers for the host entry points (cudaHostAlloc / cudaFreeHost). */
