@@ -675,6 +675,13 @@ size_t chunk_for(size_t widest_item_bytes, size_t target = size_t(64) << 20) {
     return std::max<size_t>(size_t(1) << 14, target / std::max<size_t>(1, widest_item_bytes));
 }
 
+// Budget of one chunk of a ragged batch (items, or the pattern nodes, output elements, extensions or occurrences they
+// hold). GBWT_B200_HOST_RAGGED_BUDGET=N caps it at N, so that tests cross chunk boundaries with small batches.
+uint64_t ragged_budget(uint64_t budget) {
+    if (const int cap = env_int("GBWT_B200_HOST_RAGGED_BUDGET", 0); cap > 0) return std::min<uint64_t>(budget, static_cast<uint64_t>(cap));  // tests
+    return budget;
+}
+
 // Ragged batches: items [q0, q1) such that offsets[q1] - offsets[q0] <= node_budget (at least one item).
 size_t ragged_chunk_end(const uint64_t* offsets, size_t n, size_t q0, size_t item_budget, uint64_t node_budget) {
     size_t q1 = std::min(n, q0 + item_budget);
@@ -706,8 +713,8 @@ int run_ragged(const gbwt_b200_index* ix, const uint64_t* nodes, const uint64_t*
     cudaStream_t streams[2];
     for (int i = 0; i < 2; i++) CUDA_TRY(cudaStreamCreateWithFlags(&streams[i], cudaStreamNonBlocking));
     int rc = GBWT_B200_OK;
-    const size_t item_budget = size_t(1) << 20;
-    const uint64_t node_budget = uint64_t(8) << 20;
+    const size_t item_budget = ragged_budget(size_t(1) << 20);
+    const uint64_t node_budget = ragged_budget(uint64_t(8) << 20);
     size_t chunk_index = 0;
     for (size_t q0 = 0; q0 < n && rc == GBWT_B200_OK; chunk_index++) {
         const size_t q1 = ragged_chunk_end(offsets, n, q0, item_budget, node_budget);
@@ -766,13 +773,14 @@ int run_ragged_output(const gbwt_b200_index* ix, const uint64_t* ids, size_t m, 
     if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
     size_t free_bytes = 0, total_bytes = 0;
     CUDA_TRY(cudaMemGetInfo(&free_bytes, &total_bytes));
-    const uint64_t elem_budget = std::max<uint64_t>(uint64_t(1) << 20, (free_bytes / elem_bytes) * 6 / 10);
+    const uint64_t elem_budget = ragged_budget(std::max<uint64_t>(uint64_t(1) << 20, (free_bytes / elem_bytes) * 6 / 10));
+    const size_t item_budget = ragged_budget(m);
     cudaStream_t s;
     CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     int rc = GBWT_B200_OK;
     for (size_t i0 = 0; i0 < m && rc == GBWT_B200_OK;) {
         // all chains of the chunk in one launch: a path walk is latency-bound, so concurrency is everything
-        const size_t i1 = ragged_chunk_end(out_offsets, m, i0, m, elem_budget);
+        const size_t i1 = ragged_chunk_end(out_offsets, m, i0, item_budget, elem_budget);
         const size_t count = i1 - i0;
         const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
         uint64_t *d_ids = nullptr, *d_offsets = nullptr, *d_lengths = nullptr;
@@ -1678,7 +1686,7 @@ int gbwt_b200_sequence_lengths_device(const gbwt_b200_index* ix, const uint64_t*
 int gbwt_b200_extract_device(const gbwt_b200_index* ix, const uint64_t* d_seq_ids, size_t m, const uint64_t* d_out_offsets,
                              uint64_t* d_nodes, uint64_t* d_lengths, void* stream) {
     DEVICE_ENTRY_PROLOGUE(ix);
-    if (d_nodes == nullptr || d_out_offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null output");
+    if (m > 0 && (d_nodes == nullptr || d_out_offsets == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null output");
     return launch_extract(ix, d_seq_ids, m, d_out_offsets, 0, d_nodes, d_lengths, static_cast<cudaStream_t>(stream));
 }
 
@@ -1714,7 +1722,7 @@ int gbwt_b200_extract_dna_device(const gbwt_b200_index* ix, const uint64_t* d_se
                                  const uint64_t* d_out_offsets, uint8_t* d_bytes, uint64_t* d_lengths, void* stream) {
     DEVICE_ENTRY_PROLOGUE(ix);
     if (int rc = check_graph(ix)) return rc;
-    if (d_bytes == nullptr || d_out_offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null output");
+    if (m > 0 && (d_bytes == nullptr || d_out_offsets == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null output");
     return launch_extract_dna(ix, d_seq_ids, m, d_out_offsets, 0, endmarker, d_bytes, d_lengths, static_cast<cudaStream_t>(stream));
 }
 
@@ -1830,9 +1838,10 @@ int gbwt_b200_follow(const gbwt_b200_index* ix, const gbwt_b200_bdstate* states,
     cudaStream_t s;
     CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     int rc = GBWT_B200_OK;
-    const uint64_t out_budget = uint64_t(4) << 20;  // extensions per chunk
+    const size_t item_budget = ragged_budget(size_t(1) << 20);
+    const uint64_t out_budget = ragged_budget(uint64_t(4) << 20);  // extensions per chunk
     for (size_t i0 = 0; i0 < n && rc == GBWT_B200_OK;) {
-        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, size_t(1) << 20, out_budget);
+        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, item_budget, out_budget);
         const size_t count = i1 - i0;
         const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
         gbwt_b200_bdstate *d_states = nullptr, *d_out = nullptr;
@@ -1968,8 +1977,10 @@ int gbwt_b200_locate_states(const gbwt_b200_index* ix, const gbwt_b200_state* st
     cudaStream_t s;
     CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     int rc = GBWT_B200_OK;
+    const size_t item_budget = ragged_budget(size_t(1) << 22);
+    const uint64_t out_budget = ragged_budget(uint64_t(16) << 20);  // occurrences per chunk
     for (size_t i0 = 0; i0 < n && rc == GBWT_B200_OK;) {
-        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, size_t(1) << 22, uint64_t(16) << 20);
+        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, item_budget, out_budget);
         const size_t count = i1 - i0;
         const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
         gbwt_b200_state* d_states = nullptr;

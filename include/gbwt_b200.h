@@ -28,6 +28,8 @@
  *    leave behind is the length of the sequences they have walked, kept in device memory so that later
  *    extractions can walk them from both ends. There is no CPU fallback: every query entry point runs CUDA
  *    kernels on the device chosen at creation.
+ *  - Calls that write variable-sized results to out[out_offsets[i] ..] (follow, extract, locate_states, node sequences,
+ *    DNA) write nothing outside out[out_offsets[0] .. out_offsets[n]); out_offsets[0] may be above 0.
  *  - Damaged input is rejected with GBWT_B200_E_INVALID_DATA; no C++ exception crosses this boundary.
  */
 #ifndef GBWT_B200_H
@@ -279,7 +281,13 @@ GBWT_B200_API int gbwt_b200_dna_lengths(const gbwt_b200_index* index, const uint
 GBWT_B200_API int gbwt_b200_extract_dna(const gbwt_b200_index* index, const uint64_t* seq_ids, size_t m, uint8_t endmarker,
                                        const uint64_t* out_offsets, uint8_t* bytes, uint64_t* lengths);
 
-/* ---- device-pointer entry points (inputs and outputs already resident in HBM) ------------------- */
+/* ---- device-pointer entry points (inputs and outputs already resident in HBM) -------------------
+ * Each answers like its host twin above, for the whole batch at once, on the caller's stream. Ragged offsets and output
+ * slots are absolute: pattern q is d_nodes[d_offsets[q] .. d_offsets[q+1]) and result i goes to d_out[d_out_offsets[i] ..],
+ * so d_offsets + q0 of a larger batch (d_offsets[0] > 0) searches rows q0.. of it. d_out may alias d_states in
+ * gbwt_b200_extend_device and gbwt_b200_bd_extend_device. After the checks on the index (GBWT_B200_E_NOT_BIDIRECTIONAL
+ * for the bidirectional calls and follow, GBWT_B200_E_NO_GRAPH, GBWT_B200_E_NO_SAMPLES), which launch nothing, an empty
+ * batch (n == 0 or m == 0) returns GBWT_B200_OK and launches nothing; its pointers may be NULL. */
 GBWT_B200_API int gbwt_b200_find_extend_device(const gbwt_b200_index* index, const uint64_t* d_patterns, size_t n,
                                               size_t k, gbwt_b200_state* d_out, void* stream);
 GBWT_B200_API int gbwt_b200_find_extend_u32_device(const gbwt_b200_index* index, const uint32_t* d_patterns, size_t n,
