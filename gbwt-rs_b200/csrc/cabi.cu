@@ -606,68 +606,22 @@ int launch_node_sequences(const gbwt_b200_index* ix, const uint64_t* node_ids, s
 
 // ---- host <-> device pipeline ----------------------------------------------------------------------
 
-// A fixed-size-per-item array on the host side of a batched call.
+// How an array of a batched host call is cut for the chunk of items [q0, q1).
+enum class Slice {
+    Item,      // `width` bytes per item: items q0 .. q1
+    Offsets,   // the chunking offsets themselves: words q0 .. q1, both included
+    Elements,  // `width` bytes per element: elements offsets[q0] .. offsets[q1] (pattern nodes, output slots)
+};
+
+// An array on the host side of a batched call. One with neither `in` nor `out` is device scratch.
 struct HostArray {
     const void* in;     // copied to the device before the kernel (may be null)
     void* out;          // copied back after the kernel (may be null)
-    size_t item_bytes;
+    size_t width;
+    Slice slice = Slice::Item;
+    int fill = -1;      // byte written over the device array before the kernel (-1: none), so that output slots larger
+                        // than their results carry it back to the caller, not stale pool memory
 };
-
-// Processes items [0, n) in chunks on alternating streams: H2D of the chunk's inputs, the kernel(s), D2H of its outputs.
-// With page-locked host memory the copies of one chunk overlap the kernels of the others, and the host-to-device copies
-// follow each other without a gap: the call takes the time of its input copies plus whatever is left to do when the last
-// byte has arrived. That tail is the last chunk's kernels and output copy, so the last chunk's worth of items is cut into
-// halves (1/2, 1/4, ... of a chunk, down to 1/16): the kernels of each piece run under the copy of the next, and what
-// follows the last copy is the work of a sixteenth of a chunk. (Four streams: a piece must not wait for the output copy of
-// the piece two before it.)
-// `launch(begin, count, device_ptrs, stream)` receives one device pointer per HostArray.
-template <class Launch>
-int run_chunked(const gbwt_b200_index* ix, size_t n, const std::vector<HostArray>& arrays, size_t chunk_items, Launch launch) {
-    if (n == 0) return GBWT_B200_OK;
-    DeviceScope scope(ix->device);
-    if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
-    constexpr int MAX_STREAMS = 4;
-    cudaStream_t streams[MAX_STREAMS] = {nullptr, nullptr, nullptr, nullptr};
-    const bool taper = n > chunk_items && env_int("GBWT_B200_HOST_TAPER", 1) != 0;
-    const size_t min_items = std::max<size_t>(size_t(1) << 14, chunk_items / 16);
-    const int n_streams = n > chunk_items ? (taper ? MAX_STREAMS : 2) : 1;
-    for (int i = 0; i < n_streams; i++) CUDA_TRY(cudaStreamCreateWithFlags(&streams[i], cudaStreamNonBlocking));
-    int rc = GBWT_B200_OK;
-    std::vector<void*> dptr(arrays.size(), nullptr);
-    size_t chunk_index = 0;
-    for (size_t begin = 0, count = 0; begin < n && rc == GBWT_B200_OK; begin += count, chunk_index++) {
-        const size_t left = n - begin;
-        count = std::min(chunk_items, left);
-        if (taper && left <= chunk_items && left / 2 >= min_items) count = left / 2;
-        cudaStream_t s = streams[chunk_index % n_streams];
-        for (size_t a = 0; a < arrays.size() && rc == GBWT_B200_OK; a++) {
-            cudaError_t e = cudaMallocAsync(&dptr[a], std::max<size_t>(16, count * arrays[a].item_bytes), s);
-            if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMallocAsync"); break; }
-            if (arrays[a].in != nullptr) {
-                e = cudaMemcpyAsync(dptr[a], static_cast<const char*>(arrays[a].in) + begin * arrays[a].item_bytes,
-                                    count * arrays[a].item_bytes, cudaMemcpyHostToDevice, s);
-                if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
-            }
-        }
-        if (rc == GBWT_B200_OK) rc = launch(begin, count, dptr, s);
-        for (size_t a = 0; a < arrays.size(); a++) {
-            if (dptr[a] == nullptr) continue;
-            if (rc == GBWT_B200_OK && arrays[a].out != nullptr) {
-                cudaError_t e = cudaMemcpyAsync(static_cast<char*>(arrays[a].out) + begin * arrays[a].item_bytes, dptr[a],
-                                                count * arrays[a].item_bytes, cudaMemcpyDeviceToHost, s);
-                if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
-            }
-            cudaFreeAsync(dptr[a], s);
-            dptr[a] = nullptr;
-        }
-    }
-    for (int i = 0; i < n_streams; i++) {
-        cudaError_t e = cudaStreamSynchronize(streams[i]);
-        if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-        cudaStreamDestroy(streams[i]);
-    }
-    return rc;
-}
 
 // Chunk size: about 64 MiB of the widest array per chunk, at least 16 Ki items.
 size_t chunk_for(size_t widest_item_bytes, size_t target = size_t(64) << 20) {
@@ -680,6 +634,13 @@ size_t chunk_for(size_t widest_item_bytes, size_t target = size_t(64) << 20) {
 uint64_t ragged_budget(uint64_t budget) {
     if (const int cap = env_int("GBWT_B200_HOST_RAGGED_BUDGET", 0); cap > 0) return std::min<uint64_t>(budget, static_cast<uint64_t>(cap));  // tests
     return budget;
+}
+
+// Fixed-size batches: `items` per chunk, and with `taper` the last chunk's worth cut into halves (see run_chunked).
+size_t fixed_chunk_end(size_t n, size_t q0, size_t items, bool taper) {
+    const size_t left = n - q0;
+    if (taper && left <= items && left / 2 >= std::max<size_t>(size_t(1) << 14, items / 16)) return q0 + left / 2;
+    return q0 + std::min(items, left);
 }
 
 // Ragged batches: items [q0, q1) such that offsets[q1] - offsets[q0] <= node_budget (at least one item).
@@ -701,70 +662,92 @@ bool offsets_valid(const uint64_t* offsets, size_t n) {
     return true;
 }
 
-// Uploads and launches a ragged (nodes, offsets) batch with optional per-item u64 side arrays and one output
-// array of `out_bytes` per item. `launch(d_nodes, d_offsets, base, d_side[], count, d_out, stream)`.
+// Where the chunks of a batch end, and how many streams they alternate on.
+struct Chunking {
+    size_t items;                       // items per chunk (ragged: at most)
+    int streams;
+    bool taper = false;                 // fixed-size: cut the last chunk's worth into halves
+    const uint64_t* offsets = nullptr;  // ragged: item i holds elements offsets[i] .. offsets[i+1]
+    uint64_t elems = 0;                 // ragged: elements per chunk, at most (but at least one item)
+};
+
+// Fixed-size chunks of `items` items: one stream for a batch of one chunk, two for more, four with the tapered tail.
+Chunking fixed_chunks(size_t n, size_t items) {
+    if (n <= items) return {items, 1};
+    const bool taper = env_int("GBWT_B200_HOST_TAPER", 1) != 0;
+    return {items, taper ? 4 : 2, taper};
+}
+
+// Ragged chunks of at most `items` items and `elems` elements, each capped by ragged_budget.
+Chunking ragged_chunks(const uint64_t* offsets, size_t items, uint64_t elems, int streams) {
+    return {ragged_budget(items), streams, false, offsets, ragged_budget(elems)};
+}
+
+// Processes items [0, n) in chunks on alternating streams: H2D of the chunk's inputs, the kernel(s), D2H of its outputs.
+// With page-locked host memory the copies of one chunk overlap the kernels of the others, and the host-to-device copies
+// follow each other without a gap: the call takes the time of its input copies plus whatever is left to do when the last
+// byte has arrived. That tail is the last chunk's kernels and output copy, so the last chunk's worth of items is cut into
+// halves (1/2, 1/4, ... of a chunk, down to 1/16): the kernels of each piece run under the copy of the next, and what
+// follows the last copy is the work of a sixteenth of a chunk. (Four streams: a piece must not wait for the output copy of
+// the piece two before it.)
+// `launch(q0, count, device_ptrs, stream)` receives one device pointer per HostArray. Empty slices are neither filled nor
+// copied, but still get a device array.
 template <class Launch>
-int run_ragged(const gbwt_b200_index* ix, const uint64_t* nodes, const uint64_t* offsets, size_t n,
-               const std::vector<const uint64_t*>& side, void* out, size_t out_bytes, Launch launch) {
+int run_chunked(const gbwt_b200_index* ix, size_t n, const std::vector<HostArray>& arrays, const Chunking& c, Launch launch) {
     if (n == 0) return GBWT_B200_OK;
-    if (!offsets_valid(offsets, n)) return fail(GBWT_B200_E_ARGUMENT, "offsets must be non-decreasing");
     DeviceScope scope(ix->device);
     if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
-    cudaStream_t streams[2];
-    for (int i = 0; i < 2; i++) CUDA_TRY(cudaStreamCreateWithFlags(&streams[i], cudaStreamNonBlocking));
+    std::vector<cudaStream_t> streams(c.streams, nullptr);
+    for (cudaStream_t& s : streams) CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     int rc = GBWT_B200_OK;
-    const size_t item_budget = ragged_budget(size_t(1) << 20);
-    const uint64_t node_budget = ragged_budget(uint64_t(8) << 20);
-    size_t chunk_index = 0;
-    for (size_t q0 = 0; q0 < n && rc == GBWT_B200_OK; chunk_index++) {
-        const size_t q1 = ragged_chunk_end(offsets, n, q0, item_budget, node_budget);
-        const size_t count = q1 - q0;
-        const uint64_t base = offsets[q0], n_nodes = offsets[q1] - base;
-        cudaStream_t s = streams[chunk_index % 2];
-        uint64_t *d_nodes = nullptr, *d_offsets = nullptr;
-        void* d_out = nullptr;
-        std::vector<uint64_t*> d_side(side.size(), nullptr);
-        auto alloc = [&](void** p, size_t bytes) {
-            cudaError_t e = cudaMallocAsync(p, std::max<size_t>(16, bytes), s);
-            if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaMallocAsync");
-        };
-        auto upload = [&](void* d, const void* h, size_t bytes) {
-            if (rc != GBWT_B200_OK || bytes == 0) return;
-            cudaError_t e = cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
-        };
-        alloc(reinterpret_cast<void**>(&d_nodes), n_nodes * 8);
-        alloc(reinterpret_cast<void**>(&d_offsets), (count + 1) * 8);
-        alloc(&d_out, count * out_bytes);
-        for (size_t a = 0; a < side.size(); a++) alloc(reinterpret_cast<void**>(&d_side[a]), count * 8);
-        upload(d_nodes, nodes + base, n_nodes * 8);
-        upload(d_offsets, offsets + q0, (count + 1) * 8);
-        for (size_t a = 0; a < side.size(); a++) upload(d_side[a], side[a] + q0, count * 8);
-        if (rc == GBWT_B200_OK) rc = launch(d_nodes, d_offsets, base, d_side, count, d_out, s);
-        if (rc == GBWT_B200_OK) {
-            cudaError_t e = cudaMemcpyAsync(static_cast<char*>(out) + q0 * out_bytes, d_out, count * out_bytes,
-                                            cudaMemcpyDeviceToHost, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
+    std::vector<void*> dptr(arrays.size(), nullptr);
+    std::vector<size_t> at(arrays.size()), bytes(arrays.size());  // the chunk's slice of each array on the host
+    for (size_t q0 = 0, chunk_index = 0; q0 < n && rc == GBWT_B200_OK; chunk_index++) {
+        const size_t q1 = c.offsets != nullptr ? ragged_chunk_end(c.offsets, n, q0, c.items, c.elems)
+                                               : fixed_chunk_end(n, q0, c.items, c.taper);
+        cudaStream_t s = streams[chunk_index % streams.size()];
+        for (size_t a = 0; a < arrays.size() && rc == GBWT_B200_OK; a++) {
+            const HostArray& h = arrays[a];
+            const size_t first = h.slice == Slice::Elements ? c.offsets[q0] : q0;
+            const size_t end = h.slice == Slice::Elements ? c.offsets[q1] : h.slice == Slice::Offsets ? q1 + 1 : q1;
+            at[a] = first * h.width;
+            bytes[a] = (end - first) * h.width;
+            cudaError_t e = cudaMallocAsync(&dptr[a], std::max<size_t>(16, bytes[a]), s);
+            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMallocAsync");
         }
-        if (d_nodes) cudaFreeAsync(d_nodes, s);
-        if (d_offsets) cudaFreeAsync(d_offsets, s);
-        if (d_out) cudaFreeAsync(d_out, s);
-        for (uint64_t* p : d_side) if (p) cudaFreeAsync(p, s);
+        for (size_t a = 0; a < arrays.size() && rc == GBWT_B200_OK; a++) {
+            const HostArray& h = arrays[a];
+            if (bytes[a] == 0) continue;
+            cudaError_t e = h.fill >= 0 ? cudaMemsetAsync(dptr[a], h.fill, bytes[a], s) : cudaSuccess;
+            if (e == cudaSuccess && h.in != nullptr)
+                e = cudaMemcpyAsync(dptr[a], static_cast<const char*>(h.in) + at[a], bytes[a], cudaMemcpyHostToDevice, s);
+            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
+        }
+        if (rc == GBWT_B200_OK) rc = launch(q0, q1 - q0, dptr, s);
+        for (size_t a = 0; a < arrays.size(); a++) {
+            if (dptr[a] == nullptr) continue;
+            if (rc == GBWT_B200_OK && arrays[a].out != nullptr && bytes[a] > 0) {
+                cudaError_t e = cudaMemcpyAsync(static_cast<char*>(arrays[a].out) + at[a], dptr[a], bytes[a], cudaMemcpyDeviceToHost, s);
+                if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
+            }
+            cudaFreeAsync(dptr[a], s);
+            dptr[a] = nullptr;
+        }
         q0 = q1;
     }
-    for (int i = 0; i < 2; i++) {
-        cudaError_t e = cudaStreamSynchronize(streams[i]);
+    for (cudaStream_t s : streams) {
+        cudaError_t e = cudaStreamSynchronize(s);
         if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-        cudaStreamDestroy(streams[i]);
+        cudaStreamDestroy(s);
     }
     return rc;
 }
 
-// Batches whose item i produces a variable number of `elem_bytes`-sized elements into out[offsets[i] .. offsets[i+1]):
-// ids up, results down, in chunks bounded by free HBM. `launch(d_ids, count, d_offsets, base, d_out, d_lengths, stream)`.
-template <class Launch>
-int run_ragged_output(const gbwt_b200_index* ix, const uint64_t* ids, size_t m, const uint64_t* out_offsets, void* out,
-                      size_t elem_bytes, uint64_t* lengths, Launch launch) {
+// Checks the arguments of a call that writes the `elem_bytes`-sized elements of item i into out[out_offsets[i] ..
+// out_offsets[i+1]), and sets `budget` to the elements of one chunk: 60% of the free HBM of the index's device, at least
+// 1 Mi. (Such a call puts all its items in one chunk: a path walk is latency-bound, so concurrency is everything.)
+int slot_budget(const gbwt_b200_index* ix, const uint64_t* ids, size_t m, const uint64_t* out_offsets, const void* out,
+                size_t elem_bytes, uint64_t* budget) {
     if (m == 0) return GBWT_B200_OK;
     if (ids == nullptr || out_offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null array");
     if (!offsets_valid(out_offsets, m)) return fail(GBWT_B200_E_ARGUMENT, "out_offsets must be non-decreasing");
@@ -773,48 +756,8 @@ int run_ragged_output(const gbwt_b200_index* ix, const uint64_t* ids, size_t m, 
     if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
     size_t free_bytes = 0, total_bytes = 0;
     CUDA_TRY(cudaMemGetInfo(&free_bytes, &total_bytes));
-    const uint64_t elem_budget = ragged_budget(std::max<uint64_t>(uint64_t(1) << 20, (free_bytes / elem_bytes) * 6 / 10));
-    const size_t item_budget = ragged_budget(m);
-    cudaStream_t s;
-    CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-    int rc = GBWT_B200_OK;
-    for (size_t i0 = 0; i0 < m && rc == GBWT_B200_OK;) {
-        // all chains of the chunk in one launch: a path walk is latency-bound, so concurrency is everything
-        const size_t i1 = ragged_chunk_end(out_offsets, m, i0, item_budget, elem_budget);
-        const size_t count = i1 - i0;
-        const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
-        uint64_t *d_ids = nullptr, *d_offsets = nullptr, *d_lengths = nullptr;
-        void* d_out = nullptr;
-        auto alloc = [&](void** p, size_t bytes) {
-            cudaError_t e = cudaMallocAsync(p, std::max<size_t>(16, bytes), s);
-            if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaMallocAsync");
-        };
-        alloc(reinterpret_cast<void**>(&d_ids), count * 8); alloc(reinterpret_cast<void**>(&d_offsets), (count + 1) * 8);
-        alloc(&d_out, cap * elem_bytes); alloc(reinterpret_cast<void**>(&d_lengths), count * 8);
-        if (rc == GBWT_B200_OK) {
-            // slots may be larger than the results: the slack must not carry stale pool memory back to the caller
-            cudaError_t e = cap > 0 ? cudaMemsetAsync(d_out, 0, cap * elem_bytes, s) : cudaSuccess;
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_ids, ids + i0, count * 8, cudaMemcpyHostToDevice, s);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_offsets, out_offsets + i0, (count + 1) * 8, cudaMemcpyHostToDevice, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
-        }
-        if (rc == GBWT_B200_OK) rc = launch(d_ids, count, d_offsets, base, d_out, d_lengths, s);
-        if (rc == GBWT_B200_OK) {
-            cudaError_t e = cudaSuccess;
-            if (cap > 0) e = cudaMemcpyAsync(static_cast<char*>(out) + base * elem_bytes, d_out, cap * elem_bytes, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess && lengths != nullptr) e = cudaMemcpyAsync(lengths + i0, d_lengths, count * 8, cudaMemcpyDeviceToHost, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
-        }
-        if (d_ids) cudaFreeAsync(d_ids, s);
-        if (d_offsets) cudaFreeAsync(d_offsets, s);
-        if (d_out) cudaFreeAsync(d_out, s);
-        if (d_lengths) cudaFreeAsync(d_lengths, s);
-        i0 = i1;
-    }
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-    cudaStreamDestroy(s);
-    return rc;
+    *budget = std::max<uint64_t>(uint64_t(1) << 20, (free_bytes / elem_bytes) * 6 / 10);
+    return GBWT_B200_OK;
 }
 
 int check_index(const gbwt_b200_index* ix) {
@@ -1732,7 +1675,7 @@ int gbwt_b200_find(const gbwt_b200_index* ix, const uint64_t* nodes, size_t n, g
     if (int rc = check_index(ix)) return rc;
     if (n > 0 && (nodes == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{nodes, nullptr, 8}, {nullptr, out, sizeof(gbwt_b200_state)}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_state)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_state))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_find(ix, static_cast<uint64_t*>(d[0]), count, static_cast<gbwt_b200_state*>(d[1]), s);
     });
 }
@@ -1741,7 +1684,7 @@ int gbwt_b200_extend(const gbwt_b200_index* ix, const gbwt_b200_state* states, c
     if (int rc = check_index(ix)) return rc;
     if (n > 0 && (states == nullptr || nodes == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{states, out, sizeof(gbwt_b200_state)}, {nodes, nullptr, 8}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_state)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_state))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         gbwt_b200_state* st = static_cast<gbwt_b200_state*>(d[0]);
         return launch_extend(ix, st, static_cast<uint64_t*>(d[1]), count, st, s);
     });
@@ -1753,7 +1696,7 @@ int gbwt_b200_find_extend(const gbwt_b200_index* ix, const uint64_t* patterns, s
     std::vector<HostArray> arrays = {{k > 0 ? patterns : nullptr, nullptr, 8 * k}, {nullptr, out, sizeof(gbwt_b200_state)}};
     // (pattern batches take larger chunks: a chunk is sorted and searched on its own, and the record windows of the
     // search kernel want many queries each)
-    return run_chunked(ix, n, arrays, chunk_for(std::max<size_t>(8 * k, sizeof(gbwt_b200_state)), size_t(512) << 20),
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(std::max<size_t>(8 * k, sizeof(gbwt_b200_state)), size_t(512) << 20)),
                        [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_find_extend(ix, static_cast<uint64_t*>(d[0]), count, k, static_cast<gbwt_b200_state*>(d[1]), s);
     });
@@ -1763,7 +1706,7 @@ int gbwt_b200_find_extend_u32(const gbwt_b200_index* ix, const uint32_t* pattern
     if (int rc = check_index(ix)) return rc;
     if (n > 0 && ((k > 0 && patterns == nullptr) || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{k > 0 ? patterns : nullptr, nullptr, 4 * k}, {nullptr, out, sizeof(gbwt_b200_state)}};
-    return run_chunked(ix, n, arrays, chunk_for(std::max<size_t>(4 * k, sizeof(gbwt_b200_state)), size_t(256) << 20),
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(std::max<size_t>(4 * k, sizeof(gbwt_b200_state)), size_t(256) << 20)),
                        [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_find_extend(ix, static_cast<uint32_t*>(d[0]), count, k, static_cast<gbwt_b200_state*>(d[1]), s);
     });
@@ -1772,9 +1715,14 @@ int gbwt_b200_find_extend_u32(const gbwt_b200_index* ix, const uint32_t* pattern
 int gbwt_b200_find_extend_ragged(const gbwt_b200_index* ix, const uint64_t* nodes, const uint64_t* offsets, size_t n, gbwt_b200_state* out) {
     if (int rc = check_index(ix)) return rc;
     if (n > 0 && (offsets == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
-    return run_ragged(ix, nodes, offsets, n, {}, out, sizeof(gbwt_b200_state),
-                      [&](uint64_t* d_nodes, uint64_t* d_offsets, uint64_t base, std::vector<uint64_t*>&, size_t count, void* d_out, cudaStream_t s) {
-        return launch_find_extend_ragged(ix, d_nodes, d_offsets, base, count, static_cast<gbwt_b200_state*>(d_out), s);
+    if (!offsets_valid(offsets, n)) return fail(GBWT_B200_E_ARGUMENT, "offsets must be non-decreasing");
+    if (n > 0 && nodes == nullptr && offsets[n] > offsets[0]) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    std::vector<HostArray> arrays = {{nodes, nullptr, 8, Slice::Elements}, {offsets, nullptr, 8, Slice::Offsets},
+                                     {nullptr, out, sizeof(gbwt_b200_state)}};
+    return run_chunked(ix, n, arrays, ragged_chunks(offsets, size_t(1) << 20, uint64_t(8) << 20, 2),
+                       [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_find_extend_ragged(ix, static_cast<uint64_t*>(d[0]), static_cast<uint64_t*>(d[1]), offsets[q0], count,
+                                         static_cast<gbwt_b200_state*>(d[2]), s);
     });
 }
 
@@ -1783,7 +1731,7 @@ int gbwt_b200_bd_find(const gbwt_b200_index* ix, const uint64_t* nodes, size_t n
     if (int rc = check_bidirectional(ix)) return rc;
     if (n > 0 && (nodes == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{nodes, nullptr, 8}, {nullptr, out, sizeof(gbwt_b200_bdstate)}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_bdstate)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_bdstate))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_bd_find(ix, static_cast<uint64_t*>(d[0]), count, static_cast<gbwt_b200_bdstate*>(d[1]), s);
     });
 }
@@ -1794,7 +1742,7 @@ static int bd_extend_host(const gbwt_b200_index* ix, const gbwt_b200_bdstate* st
     if (int rc = check_bidirectional(ix)) return rc;
     if (n > 0 && (states == nullptr || nodes == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{states, out, sizeof(gbwt_b200_bdstate)}, {nodes, nullptr, 8}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_bdstate)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_bdstate))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         gbwt_b200_bdstate* st = static_cast<gbwt_b200_bdstate*>(d[0]);
         return launch_bd_extend(ix, st, static_cast<uint64_t*>(d[1]), count, backward, st, s);
     });
@@ -1813,9 +1761,14 @@ int gbwt_b200_bd_search(const gbwt_b200_index* ix, const uint64_t* nodes, const 
     if (int rc = check_bidirectional(ix)) return rc;
     if (n > 0 && (offsets == nullptr || first == nullptr || start == nullptr || end == nullptr || out == nullptr))
         return fail(GBWT_B200_E_ARGUMENT, "null array");
-    return run_ragged(ix, nodes, offsets, n, {first, start, end}, out, sizeof(gbwt_b200_bdstate),
-                      [&](uint64_t* d_nodes, uint64_t* d_offsets, uint64_t base, std::vector<uint64_t*>& side, size_t count, void* d_out, cudaStream_t s) {
-        return launch_bd_search(ix, d_nodes, d_offsets, base, side[0], side[1], side[2], count, static_cast<gbwt_b200_bdstate*>(d_out), s);
+    if (!offsets_valid(offsets, n)) return fail(GBWT_B200_E_ARGUMENT, "offsets must be non-decreasing");
+    if (n > 0 && nodes == nullptr && offsets[n] > offsets[0]) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    std::vector<HostArray> arrays = {{nodes, nullptr, 8, Slice::Elements}, {offsets, nullptr, 8, Slice::Offsets},
+                                     {first, nullptr, 8}, {start, nullptr, 8}, {end, nullptr, 8}, {nullptr, out, sizeof(gbwt_b200_bdstate)}};
+    return run_chunked(ix, n, arrays, ragged_chunks(offsets, size_t(1) << 20, uint64_t(8) << 20, 2),
+                       [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        auto u = [&](int a) { return static_cast<const uint64_t*>(d[a]); };
+        return launch_bd_search(ix, u(0), u(1), offsets[q0], u(2), u(3), u(4), count, static_cast<gbwt_b200_bdstate*>(d[5]), s);
     });
 }
 
@@ -1828,61 +1781,26 @@ int gbwt_b200_follow(const gbwt_b200_index* ix, const gbwt_b200_bdstate* states,
     if (out == nullptr) {
         if (counts == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null array");
         std::vector<HostArray> arrays = {{states, nullptr, sizeof(gbwt_b200_bdstate)}, {nullptr, counts, 8}};
-        return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_bdstate)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_bdstate))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
             return launch_follow(ix, static_cast<gbwt_b200_bdstate*>(d[0]), count, backward, nullptr, 0, nullptr, static_cast<uint64_t*>(d[1]), s);
         });
     }
     if (!offsets_valid(out_offsets, n)) return fail(GBWT_B200_E_ARGUMENT, "out_offsets must be non-decreasing");
-    DeviceScope scope(ix->device);
-    if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
-    cudaStream_t s;
-    CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-    int rc = GBWT_B200_OK;
-    const size_t item_budget = ragged_budget(size_t(1) << 20);
-    const uint64_t out_budget = ragged_budget(uint64_t(4) << 20);  // extensions per chunk
-    for (size_t i0 = 0; i0 < n && rc == GBWT_B200_OK;) {
-        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, item_budget, out_budget);
-        const size_t count = i1 - i0;
-        const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
-        gbwt_b200_bdstate *d_states = nullptr, *d_out = nullptr;
-        uint64_t *d_offsets = nullptr, *d_counts = nullptr;
-        auto alloc = [&](void** p, size_t bytes) {
-            cudaError_t e = cudaMallocAsync(p, std::max<size_t>(16, bytes), s);
-            if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaMallocAsync");
-        };
-        alloc(reinterpret_cast<void**>(&d_states), count * sizeof(gbwt_b200_bdstate));
-        alloc(reinterpret_cast<void**>(&d_out), cap * sizeof(gbwt_b200_bdstate));
-        alloc(reinterpret_cast<void**>(&d_offsets), (count + 1) * 8);
-        alloc(reinterpret_cast<void**>(&d_counts), count * 8);
-        if (rc == GBWT_B200_OK) {
-            cudaError_t e = cudaMemcpyAsync(d_states, states + i0, count * sizeof(gbwt_b200_bdstate), cudaMemcpyHostToDevice, s);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_offsets, out_offsets + i0, (count + 1) * 8, cudaMemcpyHostToDevice, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
-        }
-        if (rc == GBWT_B200_OK) rc = launch_follow(ix, d_states, count, backward, d_offsets, base, d_out, d_counts, s);
-        if (rc == GBWT_B200_OK) {
-            cudaError_t e = cudaSuccess;
-            if (cap > 0) e = cudaMemcpyAsync(out + base, d_out, cap * sizeof(gbwt_b200_bdstate), cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess && counts != nullptr) e = cudaMemcpyAsync(counts + i0, d_counts, count * 8, cudaMemcpyDeviceToHost, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
-        }
-        if (d_states) cudaFreeAsync(d_states, s);
-        if (d_out) cudaFreeAsync(d_out, s);
-        if (d_offsets) cudaFreeAsync(d_offsets, s);
-        if (d_counts) cudaFreeAsync(d_counts, s);
-        i0 = i1;
-    }
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-    cudaStreamDestroy(s);
-    return rc;
+    // (no fill: what a slot holds beyond its result is unspecified, and clearing it would cost a memset per call)
+    std::vector<HostArray> arrays = {{states, nullptr, sizeof(gbwt_b200_bdstate)}, {nullptr, out, sizeof(gbwt_b200_bdstate), Slice::Elements},
+                                     {out_offsets, nullptr, 8, Slice::Offsets}, {nullptr, counts, 8}};
+    return run_chunked(ix, n, arrays, ragged_chunks(out_offsets, size_t(1) << 20, uint64_t(4) << 20, 1),
+                       [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_follow(ix, static_cast<gbwt_b200_bdstate*>(d[0]), count, backward, static_cast<uint64_t*>(d[2]), out_offsets[q0],
+                             static_cast<gbwt_b200_bdstate*>(d[1]), static_cast<uint64_t*>(d[3]), s);
+    });
 }
 
 int gbwt_b200_start(const gbwt_b200_index* ix, const uint64_t* seq_ids, size_t n, gbwt_b200_pos* out) {
     if (int rc = check_index(ix)) return rc;
     if (n > 0 && (seq_ids == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{seq_ids, nullptr, 8}, {nullptr, out, sizeof(gbwt_b200_pos)}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_pos)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_pos))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_start(ix, static_cast<uint64_t*>(d[0]), count, static_cast<gbwt_b200_pos*>(d[1]), s);
     });
 }
@@ -1895,7 +1813,7 @@ static int step_host(const gbwt_b200_index* ix, const gbwt_b200_pos* positions, 
     }
     if (n > 0 && (positions == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{positions, out, sizeof(gbwt_b200_pos)}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_pos)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_pos))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         gbwt_b200_pos* p = static_cast<gbwt_b200_pos*>(d[0]);
         return backward ? launch_backward(ix, p, count, p, s) : launch_forward(ix, p, count, p, s);
     });
@@ -1913,7 +1831,7 @@ int gbwt_b200_sequence_lengths(const gbwt_b200_index* ix, const uint64_t* seq_id
     if (m > 0 && (seq_ids == nullptr || lengths == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{seq_ids, nullptr, 8}, {nullptr, lengths, 8}};
     // all chains of the batch in one launch: a path walk is latency-bound, so concurrency is everything
-    return run_chunked(ix, m, arrays, std::max<size_t>(m, 1), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, m, arrays, fixed_chunks(m, std::max<size_t>(m, 1)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_extract(ix, static_cast<uint64_t*>(d[0]), count, nullptr, 0, nullptr, static_cast<uint64_t*>(d[1]), s);
     });
 }
@@ -1921,10 +1839,14 @@ int gbwt_b200_sequence_lengths(const gbwt_b200_index* ix, const uint64_t* seq_id
 int gbwt_b200_extract(const gbwt_b200_index* ix, const uint64_t* seq_ids, size_t m, const uint64_t* out_offsets, uint64_t* nodes,
                       uint64_t* lengths) {
     if (int rc = check_index(ix)) return rc;
-    return run_ragged_output(ix, seq_ids, m, out_offsets, nodes, sizeof(uint64_t), lengths,
-                             [&](const uint64_t* d_ids, size_t count, const uint64_t* d_offsets, uint64_t base, void* d_out, uint64_t* d_lengths, cudaStream_t s) {
-                                 return launch_extract(ix, d_ids, count, d_offsets, base, static_cast<uint64_t*>(d_out), d_lengths, s);
-                             });
+    uint64_t elems = 0;
+    if (int rc = slot_budget(ix, seq_ids, m, out_offsets, nodes, sizeof(uint64_t), &elems)) return rc;
+    std::vector<HostArray> arrays = {{seq_ids, nullptr, 8}, {nullptr, nodes, sizeof(uint64_t), Slice::Elements, 0x00},
+                                     {out_offsets, nullptr, 8, Slice::Offsets}, {nullptr, lengths, 8}};
+    return run_chunked(ix, m, arrays, ragged_chunks(out_offsets, m, elems, 1), [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_extract(ix, static_cast<uint64_t*>(d[0]), count, static_cast<uint64_t*>(d[2]), out_offsets[q0],
+                              static_cast<uint64_t*>(d[1]), static_cast<uint64_t*>(d[3]), s);
+    });
 }
 
 int gbwt_b200_dna_lengths(const gbwt_b200_index* ix, const uint64_t* seq_ids, size_t m, uint64_t* lengths) {
@@ -1932,7 +1854,7 @@ int gbwt_b200_dna_lengths(const gbwt_b200_index* ix, const uint64_t* seq_ids, si
     if (int rc = check_graph(ix)) return rc;
     if (m > 0 && (seq_ids == nullptr || lengths == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{seq_ids, nullptr, 8}, {nullptr, lengths, 8}};
-    return run_chunked(ix, m, arrays, std::max<size_t>(m, 1), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, m, arrays, fixed_chunks(m, std::max<size_t>(m, 1)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_extract_dna(ix, static_cast<uint64_t*>(d[0]), count, nullptr, 0, 0, nullptr, static_cast<uint64_t*>(d[1]), s);
     });
 }
@@ -1941,10 +1863,14 @@ int gbwt_b200_extract_dna(const gbwt_b200_index* ix, const uint64_t* seq_ids, si
                           uint8_t* bytes, uint64_t* lengths) {
     if (int rc = check_index(ix)) return rc;
     if (int rc = check_graph(ix)) return rc;
-    return run_ragged_output(ix, seq_ids, m, out_offsets, bytes, 1, lengths,
-                             [&](const uint64_t* d_ids, size_t count, const uint64_t* d_offsets, uint64_t base, void* d_out, uint64_t* d_lengths, cudaStream_t s) {
-                                 return launch_extract_dna(ix, d_ids, count, d_offsets, base, endmarker, static_cast<uint8_t*>(d_out), d_lengths, s);
-                             });
+    uint64_t elems = 0;
+    if (int rc = slot_budget(ix, seq_ids, m, out_offsets, bytes, 1, &elems)) return rc;
+    std::vector<HostArray> arrays = {{seq_ids, nullptr, 8}, {nullptr, bytes, 1, Slice::Elements, 0x00},
+                                     {out_offsets, nullptr, 8, Slice::Offsets}, {nullptr, lengths, 8}};
+    return run_chunked(ix, m, arrays, ragged_chunks(out_offsets, m, elems, 1), [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_extract_dna(ix, static_cast<uint64_t*>(d[0]), count, static_cast<uint64_t*>(d[2]), out_offsets[q0], endmarker,
+                                  static_cast<uint8_t*>(d[1]), static_cast<uint64_t*>(d[3]), s);
+    });
 }
 
 int gbwt_b200_locate(const gbwt_b200_index* ix, const gbwt_b200_pos* positions, size_t n, gbwt_b200_occurrence* out) {
@@ -1952,12 +1878,11 @@ int gbwt_b200_locate(const gbwt_b200_index* ix, const gbwt_b200_pos* positions, 
     if (int rc = check_samples(ix)) return rc;
     if (n > 0 && (positions == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{positions, nullptr, sizeof(gbwt_b200_pos)}, {nullptr, out, sizeof(gbwt_b200_occurrence)}};
-    return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_pos)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_pos))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_locate_positions(ix, static_cast<gbwt_b200_pos*>(d[0]), count, static_cast<gbwt_b200_occurrence*>(d[1]), s);
     });
 }
 
-// Chunks of states whose output slots hold at most 16 Mi occurrences (at least one state), like gbwt_b200_follow.
 int gbwt_b200_locate_states(const gbwt_b200_index* ix, const gbwt_b200_state* states, size_t n, const uint64_t* out_offsets,
                             gbwt_b200_occurrence* out, uint64_t* counts) {
     if (int rc = check_index(ix)) return rc;
@@ -1967,57 +1892,18 @@ int gbwt_b200_locate_states(const gbwt_b200_index* ix, const gbwt_b200_state* st
     if (out == nullptr) {
         if (counts == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null array");
         std::vector<HostArray> arrays = {{states, nullptr, sizeof(gbwt_b200_state)}, {nullptr, counts, 8}};
-        return run_chunked(ix, n, arrays, chunk_for(sizeof(gbwt_b200_state)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_state))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
             return launch_locate_state_batch(ix, static_cast<gbwt_b200_state*>(d[0]), count, nullptr, 0, nullptr, static_cast<uint64_t*>(d[1]), s);
         });
     }
     if (!offsets_valid(out_offsets, n)) return fail(GBWT_B200_E_ARGUMENT, "out_offsets must be non-decreasing");
-    DeviceScope scope(ix->device);
-    if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
-    cudaStream_t s;
-    CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-    int rc = GBWT_B200_OK;
-    const size_t item_budget = ragged_budget(size_t(1) << 22);
-    const uint64_t out_budget = ragged_budget(uint64_t(16) << 20);  // occurrences per chunk
-    for (size_t i0 = 0; i0 < n && rc == GBWT_B200_OK;) {
-        const size_t i1 = ragged_chunk_end(out_offsets, n, i0, item_budget, out_budget);
-        const size_t count = i1 - i0;
-        const uint64_t base = out_offsets[i0], cap = out_offsets[i1] - base;
-        gbwt_b200_state* d_states = nullptr;
-        gbwt_b200_occurrence* d_out = nullptr;
-        uint64_t *d_offsets = nullptr, *d_counts = nullptr;
-        auto alloc = [&](void** p, size_t bytes) {
-            cudaError_t e = cudaMallocAsync(p, std::max<size_t>(16, bytes), s);
-            if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaMallocAsync");
-        };
-        alloc(reinterpret_cast<void**>(&d_states), count * sizeof(gbwt_b200_state));
-        alloc(reinterpret_cast<void**>(&d_out), cap * sizeof(gbwt_b200_occurrence));
-        alloc(reinterpret_cast<void**>(&d_offsets), (count + 1) * 8);
-        alloc(reinterpret_cast<void**>(&d_counts), count * 8);
-        if (rc == GBWT_B200_OK) {
-            // slots may be larger than the answers: the slack must not carry stale pool memory back to the caller
-            cudaError_t e = cap > 0 ? cudaMemsetAsync(d_out, 0xFF, cap * sizeof(gbwt_b200_occurrence), s) : cudaSuccess;
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_states, states + i0, count * sizeof(gbwt_b200_state), cudaMemcpyHostToDevice, s);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_offsets, out_offsets + i0, (count + 1) * 8, cudaMemcpyHostToDevice, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync H2D");
-        }
-        if (rc == GBWT_B200_OK) rc = launch_locate_state_batch(ix, d_states, count, d_offsets, base, d_out, d_counts, s);
-        if (rc == GBWT_B200_OK) {
-            cudaError_t e = cudaSuccess;
-            if (cap > 0) e = cudaMemcpyAsync(out + base, d_out, cap * sizeof(gbwt_b200_occurrence), cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess && counts != nullptr) e = cudaMemcpyAsync(counts + i0, d_counts, count * 8, cudaMemcpyDeviceToHost, s);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync D2H");
-        }
-        if (d_states) cudaFreeAsync(d_states, s);
-        if (d_out) cudaFreeAsync(d_out, s);
-        if (d_offsets) cudaFreeAsync(d_offsets, s);
-        if (d_counts) cudaFreeAsync(d_counts, s);
-        i0 = i1;
-    }
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess && rc == GBWT_B200_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-    cudaStreamDestroy(s);
-    return rc;
+    std::vector<HostArray> arrays = {{states, nullptr, sizeof(gbwt_b200_state)}, {nullptr, out, sizeof(gbwt_b200_occurrence), Slice::Elements, 0xFF},
+                                     {out_offsets, nullptr, 8, Slice::Offsets}, {nullptr, counts, 8}};
+    return run_chunked(ix, n, arrays, ragged_chunks(out_offsets, size_t(1) << 22, uint64_t(16) << 20, 1),
+                       [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_locate_state_batch(ix, static_cast<gbwt_b200_state*>(d[0]), count, static_cast<uint64_t*>(d[2]), out_offsets[q0],
+                                         static_cast<gbwt_b200_occurrence*>(d[1]), static_cast<uint64_t*>(d[3]), s);
+    });
 }
 
 int gbwt_b200_node_sequence_lengths(const gbwt_b200_index* ix, const uint64_t* node_ids, size_t n, uint64_t* lengths) {
@@ -2025,7 +1911,7 @@ int gbwt_b200_node_sequence_lengths(const gbwt_b200_index* ix, const uint64_t* n
     if (int rc = check_graph(ix)) return rc;
     if (n > 0 && (node_ids == nullptr || lengths == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
     std::vector<HostArray> arrays = {{node_ids, nullptr, 8}, {nullptr, lengths, 8}};
-    return run_chunked(ix, n, arrays, chunk_for(16), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(16)), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
         return launch_node_sequences(ix, static_cast<uint64_t*>(d[0]), count, nullptr, 0, nullptr, static_cast<uint64_t*>(d[1]), s);
     });
 }
@@ -2034,10 +1920,14 @@ int gbwt_b200_node_sequences(const gbwt_b200_index* ix, const uint64_t* node_ids
                              uint64_t* lengths) {
     if (int rc = check_index(ix)) return rc;
     if (int rc = check_graph(ix)) return rc;
-    return run_ragged_output(ix, node_ids, n, out_offsets, bytes, 1, lengths,
-                             [&](const uint64_t* d_ids, size_t count, const uint64_t* d_offsets, uint64_t base, void* d_out, uint64_t* d_lengths, cudaStream_t s) {
-                                 return launch_node_sequences(ix, d_ids, count, d_offsets, base, static_cast<uint8_t*>(d_out), d_lengths, s);
-                             });
+    uint64_t elems = 0;
+    if (int rc = slot_budget(ix, node_ids, n, out_offsets, bytes, 1, &elems)) return rc;
+    std::vector<HostArray> arrays = {{node_ids, nullptr, 8}, {nullptr, bytes, 1, Slice::Elements, 0x00},
+                                     {out_offsets, nullptr, 8, Slice::Offsets}, {nullptr, lengths, 8}};
+    return run_chunked(ix, n, arrays, ragged_chunks(out_offsets, n, elems, 1), [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_node_sequences(ix, static_cast<uint64_t*>(d[0]), count, static_cast<uint64_t*>(d[2]), out_offsets[q0],
+                                     static_cast<uint8_t*>(d[1]), static_cast<uint64_t*>(d[3]), s);
+    });
 }
 
 // ---- utilities ---------------------------------------------------------------------------------------
