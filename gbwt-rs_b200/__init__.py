@@ -121,6 +121,12 @@ def _load_library() -> C.CDLL:
         "gbwt_b200_extract_dna": (i, [p, p, sz, C.c_uint8, p, p, p]),
         "gbwt_b200_dna_lengths_device": (i, [p, p, sz, p, p]),
         "gbwt_b200_extract_dna_device": (i, [p, p, sz, C.c_uint8, p, p, p, p]),
+        "gbwt_b200_seek": (i, [p, p, p, sz, p]),
+        "gbwt_b200_extract_ranges": (i, [p, p, p, p, sz, p, p, p]),
+        "gbwt_b200_extract_dna_ranges": (i, [p, p, p, p, sz, p, p, p]),
+        "gbwt_b200_seek_device": (i, [p, p, p, sz, p, p]),
+        "gbwt_b200_extract_ranges_device": (i, [p, p, p, p, sz, p, p, p, p]),
+        "gbwt_b200_extract_dna_ranges_device": (i, [p, p, p, p, sz, p, p, p, p]),
         "gbwt_b200_host_alloc": (p, [sz]), "gbwt_b200_host_free": (None, [p]),
         "gbwt_b200_kernel_launches": (u64, []), "gbwt_b200_version": (C.c_char_p, []),
     }
@@ -554,6 +560,57 @@ class GBWT:
         _lib.gbwt_b200_locate_info(self._h, _ptr(raw))
         keys = ("present", "interval", "samples", "bytes", "build_us", "lf_steps")
         return {k: int(v) for k, v in zip(keys, raw)}
+
+    # -- ranges of sequences (beyond the crate; include/gbwt_b200_ranges.h) --
+    def seek(self, seq_ids, indexes=None):
+        """Position of node number j of GBWT::sequence(s) (start(s) and j forward steps). seek(s, j) returns a Pos or None;
+        with arrays, a POS_DTYPE array ({0, 0} where s >= sequences() or j >= the length of s)."""
+        if _is_scalar(seq_ids):
+            r = self.seek(np.array([seq_ids], dtype=np.uint64), np.array([indexes], dtype=np.uint64))[0]
+            return Pos(int(r["node"]), int(r["offset"])) if r["node"] != ENDMARKER else None
+        ids, idx = _u64(seq_ids), _u64(indexes)
+        if len(ids) != len(idx):
+            raise ValueError("seq_ids and indexes must have the same length")
+        out = np.zeros(len(ids), POS_DTYPE)
+        self._check(_lib.gbwt_b200_seek(self._h, _ptr(ids), _ptr(idx), len(ids), _ptr(out)))
+        return out
+
+    def _ranges(self, fn, full, seq_ids, starts, ends, dtype):
+        ids, starts, ends = _u64(seq_ids), _u64(starts), _u64(ends)
+        if not len(ids) == len(starts) == len(ends):
+            raise ValueError("seq_ids, starts and ends must have the same length")
+        full = np.where(full == _U64MAX, np.uint64(0), full)
+        stop = np.minimum(ends, full)
+        sizes = np.where(stop > starts, stop - starts, np.uint64(0)).astype(np.uint64)
+        offsets = np.zeros(len(ids) + 1, np.uint64)
+        np.cumsum(sizes, out=offsets[1:])
+        data = np.zeros(int(offsets[-1]), dtype)
+        got = np.zeros(len(ids), np.uint64)
+        self._check(fn(self._h, _ptr(ids), _ptr(starts), _ptr(ends), len(ids), _ptr(offsets), _ptr(data), _ptr(got)))
+        return offsets, data, got
+
+    def extract_ranges(self, seq_ids, starts, ends):
+        """extract(s)[start:min(end, len)] for many (s, start, end): (offsets, nodes, lengths) shaped like extract; lengths[i] =
+        max(0, min(end, len) - start), UINT64_MAX where the sequence is None."""
+        return self._ranges(_lib.gbwt_b200_extract_ranges, self.sequence_lengths(seq_ids), seq_ids, starts, ends, np.uint64)
+
+    def extract_dna_ranges(self, seq_ids, starts, ends):
+        """Bytes [start, min(end, L)) of extract_dna(s) without its endmarker (L = dna_lengths(s) - 1), for many (s, start, end):
+        (offsets, bytes, lengths) shaped like extract_dna."""
+        full = self.dna_lengths(seq_ids)
+        full = np.where(full == _U64MAX, full, full - np.uint64(1))
+        return self._ranges(_lib.gbwt_b200_extract_dna_ranges, full, seq_ids, starts, ends, np.uint8)
+
+    def seek_device(self, d_ids: int, d_indexes: int, n: int, d_out: int, stream: int = 0):
+        self._check(_lib.gbwt_b200_seek_device(self._h, d_ids, d_indexes, n, d_out, stream))
+
+    def extract_ranges_device(self, d_ids: int, d_starts: int, d_ends: int, m: int, d_out_offsets: int, d_nodes: int, d_lengths: int,
+                              stream: int = 0):
+        self._check(_lib.gbwt_b200_extract_ranges_device(self._h, d_ids, d_starts, d_ends, m, d_out_offsets, d_nodes, d_lengths, stream))
+
+    def extract_dna_ranges_device(self, d_ids: int, d_starts: int, d_ends: int, m: int, d_out_offsets: int, d_bytes: int, d_lengths: int,
+                                  stream: int = 0):
+        self._check(_lib.gbwt_b200_extract_dna_ranges_device(self._h, d_ids, d_starts, d_ends, m, d_out_offsets, d_bytes, d_lengths, stream))
 
     # -- node sequences and DNA-level extraction (GBZ files; src/gbz.rs:286-306, src/bin/gbz-extract.rs:173-189) --
     def has_graph(self) -> bool: return bool(_lib.gbwt_b200_has_graph(self._h))

@@ -16,12 +16,14 @@
 #include <vector>
 
 #include "../../include/gbwt_b200.h"
+#include "../../include/gbwt_b200_ranges.h"
 #include "find_mixed.h"
 #include "find_window.h"
 #include "kernels.cuh"
 #include "layout_builder.h"
 #include "layout_writer.h"
 #include "locate.h"
+#include "ranges.h"
 #include "sds_loader.h"
 
 using namespace gbwt_b200;
@@ -861,6 +863,67 @@ int check_graph(const gbwt_b200_index* ix) {
     return GBWT_B200_OK;
 }
 
+// The path checkpoints the range walks start from (ranges.h): table == nullptr where the index has none, and for DNA where it
+// has no DNA checkpoints (or GBWT_B200_DNA_CHECKPOINTS=0, as in launch_extract_dna).
+CheckpointView range_view(const gbwt_b200_index* ix, bool dna) {
+    CheckpointView cv = ix->ckpt;
+    if (!ix->ckpt_ok || (dna && !(ix->dna_ckpt_ok && env_int("GBWT_B200_DNA_CHECKPOINTS", 1) != 0))) cv.table = nullptr;
+    return cv;
+}
+
+int launch_seek_batch(const gbwt_b200_index* ix, const uint64_t* ids, const uint64_t* indexes, size_t n, gbwt_b200_pos* out, cudaStream_t s) {
+    if (n == 0) return GBWT_B200_OK;
+    const cudaError_t e = launch_seek(ix->view, range_view(ix, false), ix->ckpt_shift, ids, indexes, n, out, ix->sm_count, s);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return e == cudaSuccess ? GBWT_B200_OK : cuda_fail(e, "k_seek");
+}
+
+int launch_range_batch(const gbwt_b200_index* ix, bool dna, const uint64_t* ids, const uint64_t* starts, const uint64_t* ends, size_t m,
+                       const uint64_t* out_offsets, uint64_t base, void* out, uint64_t* lengths, cudaStream_t s) {
+    if (m == 0) return GBWT_B200_OK;
+    const CheckpointView cv = range_view(ix, dna);
+    const cudaError_t e = dna ? launch_range_dna(ix->view, ix->graph, cv, static_cast<const uint64_t*>(ix->d_ckpt_dna),
+                                                 static_cast<const uint64_t*>(ix->d_dna_len), ids, starts, ends, m, out_offsets, base,
+                                                 static_cast<uint8_t*>(out), lengths, ix->sm_count, s)
+                              : launch_range_nodes(ix->view, cv, ix->ckpt_shift, ids, starts, ends, m, out_offsets, base,
+                                                   static_cast<uint64_t*>(out), lengths, ix->sm_count, s);
+    g_launches.fetch_add(4, std::memory_order_relaxed);  // (the plan, CUB's two scan kernels, the pieces)
+    return e == cudaSuccess ? GBWT_B200_OK : cuda_fail(e, dna ? "k_range_pieces<true>" : "k_range_pieces<false>");
+}
+
+// Host twin of the range calls: the arguments checked like extract's, then the chunk loop over the output slots.
+int ranges_host(const gbwt_b200_index* ix, bool dna, const uint64_t* ids, const uint64_t* starts, const uint64_t* ends, size_t m,
+                const uint64_t* out_offsets, void* out, uint64_t* lengths) {
+    if (int rc = check_index(ix)) return rc;
+    if (dna) { if (int rc = check_graph(ix)) return rc; }
+    const size_t width = dna ? 1 : sizeof(uint64_t);
+    uint64_t elems = 0;
+    if (int rc = slot_budget(ix, ids, m, out_offsets, out, width, &elems)) return rc;
+    if (m > 0 && (starts == nullptr || ends == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    std::vector<HostArray> arrays = {{ids, nullptr, 8}, {starts, nullptr, 8}, {ends, nullptr, 8}, {nullptr, out, width, Slice::Elements, 0x00},
+                                     {out_offsets, nullptr, 8, Slice::Offsets}, {nullptr, lengths, 8}};
+    return run_chunked(ix, m, arrays, ragged_chunks(out_offsets, m, elems, 1), [&](size_t q0, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        auto u = [&](int a) { return static_cast<const uint64_t*>(d[a]); };
+        return launch_range_batch(ix, dna, u(0), u(1), u(2), count, u(4), out_offsets[q0], d[3], static_cast<uint64_t*>(d[5]), s);
+    });
+}
+
+// Device twin: the batch in slices of 2^30 ranges (the scan of a slice is indexed with 64-bit CUB offsets; slices keep each
+// launch's temporary arrays bounded).
+int ranges_device(const gbwt_b200_index* ix, bool dna, const uint64_t* ids, const uint64_t* starts, const uint64_t* ends, size_t m,
+                  const uint64_t* out_offsets, void* out, uint64_t* lengths, cudaStream_t s) {
+    if (m > 0 && (ids == nullptr || starts == nullptr || ends == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    if (m > 0 && (out == nullptr || out_offsets == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null output");
+    const size_t chunk = size_t(1) << 30;
+    for (size_t begin = 0; begin < m; begin += chunk) {
+        const size_t count = std::min(chunk, m - begin);
+        int rc = launch_range_batch(ix, dna, ids + begin, starts + begin, ends + begin, count, out_offsets + begin, 0, out,
+                                    lengths != nullptr ? lengths + begin : nullptr, s);
+        if (rc != GBWT_B200_OK) return rc;
+    }
+    return GBWT_B200_OK;
+}
+
 // In-place inclusive scan of counts[0 .. m) on stream s (the three launches of kernels.cuh).
 int scan_counts(uint32_t* counts, uint32_t m, cudaStream_t s) {
     const uint32_t tiles = (m + SCAN_TILE - 1) / SCAN_TILE;
@@ -1656,6 +1719,24 @@ int gbwt_b200_locate_states_device(const gbwt_b200_index* ix, const gbwt_b200_st
     return GBWT_B200_OK;
 }
 
+int gbwt_b200_seek_device(const gbwt_b200_index* ix, const uint64_t* d_seq_ids, const uint64_t* d_indexes, size_t n, gbwt_b200_pos* d_out,
+                          void* stream) {
+    DEVICE_ENTRY_PROLOGUE(ix);
+    if (n > 0 && (d_seq_ids == nullptr || d_indexes == nullptr || d_out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    return launch_seek_batch(ix, d_seq_ids, d_indexes, n, d_out, static_cast<cudaStream_t>(stream));
+}
+int gbwt_b200_extract_ranges_device(const gbwt_b200_index* ix, const uint64_t* d_seq_ids, const uint64_t* d_starts, const uint64_t* d_ends,
+                                    size_t m, const uint64_t* d_out_offsets, uint64_t* d_nodes, uint64_t* d_lengths, void* stream) {
+    DEVICE_ENTRY_PROLOGUE(ix);
+    return ranges_device(ix, false, d_seq_ids, d_starts, d_ends, m, d_out_offsets, d_nodes, d_lengths, static_cast<cudaStream_t>(stream));
+}
+int gbwt_b200_extract_dna_ranges_device(const gbwt_b200_index* ix, const uint64_t* d_seq_ids, const uint64_t* d_starts, const uint64_t* d_ends,
+                                        size_t m, const uint64_t* d_out_offsets, uint8_t* d_bytes, uint64_t* d_lengths, void* stream) {
+    DEVICE_ENTRY_PROLOGUE(ix);
+    if (int rc = check_graph(ix)) return rc;
+    return ranges_device(ix, true, d_seq_ids, d_starts, d_ends, m, d_out_offsets, d_bytes, d_lengths, static_cast<cudaStream_t>(stream));
+}
+
 int gbwt_b200_dna_lengths_device(const gbwt_b200_index* ix, const uint64_t* d_seq_ids, size_t m, uint64_t* d_lengths, void* stream) {
     DEVICE_ENTRY_PROLOGUE(ix);
     if (int rc = check_graph(ix)) return rc;
@@ -1904,6 +1985,25 @@ int gbwt_b200_locate_states(const gbwt_b200_index* ix, const gbwt_b200_state* st
         return launch_locate_state_batch(ix, static_cast<gbwt_b200_state*>(d[0]), count, static_cast<uint64_t*>(d[2]), out_offsets[q0],
                                          static_cast<gbwt_b200_occurrence*>(d[1]), static_cast<uint64_t*>(d[3]), s);
     });
+}
+
+int gbwt_b200_seek(const gbwt_b200_index* ix, const uint64_t* seq_ids, const uint64_t* indexes, size_t n, gbwt_b200_pos* out) {
+    if (int rc = check_index(ix)) return rc;
+    if (n > 0 && (seq_ids == nullptr || indexes == nullptr || out == nullptr)) return fail(GBWT_B200_E_ARGUMENT, "null array");
+    std::vector<HostArray> arrays = {{seq_ids, nullptr, 8}, {indexes, nullptr, 8}, {nullptr, out, sizeof(gbwt_b200_pos)}};
+    return run_chunked(ix, n, arrays, fixed_chunks(n, chunk_for(sizeof(gbwt_b200_pos))), [&](size_t, size_t count, std::vector<void*>& d, cudaStream_t s) {
+        return launch_seek_batch(ix, static_cast<uint64_t*>(d[0]), static_cast<uint64_t*>(d[1]), count, static_cast<gbwt_b200_pos*>(d[2]), s);
+    });
+}
+
+int gbwt_b200_extract_ranges(const gbwt_b200_index* ix, const uint64_t* seq_ids, const uint64_t* starts, const uint64_t* ends, size_t m,
+                             const uint64_t* out_offsets, uint64_t* nodes, uint64_t* lengths) {
+    return ranges_host(ix, false, seq_ids, starts, ends, m, out_offsets, nodes, lengths);
+}
+
+int gbwt_b200_extract_dna_ranges(const gbwt_b200_index* ix, const uint64_t* seq_ids, const uint64_t* starts, const uint64_t* ends, size_t m,
+                                 const uint64_t* out_offsets, uint8_t* bytes, uint64_t* lengths) {
+    return ranges_host(ix, true, seq_ids, starts, ends, m, out_offsets, bytes, lengths);
 }
 
 int gbwt_b200_node_sequence_lengths(const gbwt_b200_index* ix, const uint64_t* node_ids, size_t n, uint64_t* lengths) {

@@ -500,24 +500,7 @@ struct HalfSink {
     __device__ __forceinline__ void finish() {}
 };
 
-// Node labels of the graph in HBM: label i = bytes[starts[i] .. starts[i + 1]) (Graph::sequence, src/graph.rs:124-126).
-struct GraphView {
-    const uint64_t* starts;  // [sequences + 1]
-    const uint8_t* bytes;
-    uint64_t sequences;
-};
-
-// support::COMPLEMENT, src/support.rs:87-98, as arithmetic (a 256-entry table indexed per lane would serialise in
-// the constant cache): both cases of A/C/G/T map to the upper-case complement, every other byte to 'N'.
-__device__ __forceinline__ uint32_t complement_base(uint32_t c) {
-    const uint32_t u = c & 0xDFu;  // 'a'..'z' -> 'A'..'Z'; no other byte lands on A, C, G or T
-    uint32_t r = 'N';
-    r = (u == 'A') ? 'T' : r;
-    r = (u == 'C') ? 'G' : r;
-    r = (u == 'G') ? 'C' : r;
-    r = (u == 'T') ? 'A' : r;
-    return r;
-}
+// (struct GraphView: layout.h; complement_base: record_scan.cuh)
 
 // extract_sequence (src/bin/gbz-extract.rs:173-189): the labels of the visited nodes, reverse-complemented for
 // reverse-oriented nodes (support::reverse_complement, src/support.rs:104-110). Per group of 32 nodes every lane

@@ -128,6 +128,13 @@ struct CheckpointView {
     uint32_t lookahead;        // records ahead of the walks at which a warp touches the index once per round (0 = off)
 };
 
+// Node labels of the graph in HBM: label i = bytes[starts[i] .. starts[i + 1]) (Graph::sequence, src/graph.rs:124-126).
+struct GraphView {
+    const uint64_t* starts;  // [sequences + 1]
+    const uint8_t* bytes;
+    uint64_t sequences;
+};
+
 // Locate samples (kernels.cuh: k_build_locate, locate.cu): (sequence, index) at some positions of every sequence, indexed
 // by BWT position. The samples of record r are samples[first[r] .. first[r + 1]), sorted by offset.
 struct LocateSample { uint32_t offset, seq; uint64_t index; };  // position (record, offset) is node `index` of sequence `seq`

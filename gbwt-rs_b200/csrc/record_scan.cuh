@@ -1144,4 +1144,66 @@ GBWT_HD bool gbwt_locate(const IndexView& ix, const LocateView& lv, uint64_t nod
     }
 }
 
+// ---- ranges of sequences (gbwt_b200_ranges.h) ----------------------------------------------------------------------
+
+// support::COMPLEMENT, src/support.rs:87-98, as arithmetic (a 256-entry table indexed per lane would serialise in
+// the constant cache): both cases of A/C/G/T map to the upper-case complement, every other byte to 'N'.
+GBWT_HD uint32_t complement_base(uint32_t c) {
+    const uint32_t u = c & 0xDFu;  // 'a'..'z' -> 'A'..'Z'; no other byte lands on A, C, G or T
+    uint32_t r = 'N';
+    r = (u == 'A') ? 'T' : r;
+    r = (u == 'C') ? 'G' : r;
+    r = (u == 'G') ? 'C' : r;
+    r = (u == 'T') ? 'A' : r;
+    return r;
+}
+
+// The path checkpoint (CheckpointView) a walk to node number j of sequence s starts from, as a slot of the table. Slot k
+// of a sequence holds the first flush of the build walk at or after node k 2^shift, which is at most 31 nodes later
+// (flushes are at most 32 nodes apart, intervals at least 64): so it is slot min(j >> shift, count - 1), or the one before
+// when that one lies beyond j. The caller has checked j < seq_len[s], so the sequence has slot 0 (node 0).
+GBWT_HD uint32_t checkpoint_slot(const CheckpointView& cv, uint32_t shift, uint64_t s, uint64_t j) {
+    const uint32_t first = GBWT_LDG(cv.first + s), count = GBWT_LDG(cv.first + s + 1) - first;
+    uint64_t k = j >> shift;
+    if (k >= count) k = count - 1;
+    if (k > 0 && GBWT_LDG(&cv.table[first + k].index) > j) k--;
+    return first + static_cast<uint32_t>(k);
+}
+
+// Position of the checkpoint in `slot`; `index` receives its node number.
+GBWT_HD gbwt_b200_pos checkpoint_pos(const CheckpointView& cv, uint32_t slot, uint64_t& index) {
+    gbwt_b200_pos p;
+    p.node = GBWT_LDG(&cv.table[slot].node);
+    p.offset = GBWT_LDG(&cv.table[slot].offset);
+    index = GBWT_LDG(&cv.table[slot].index);
+    return p;
+}
+
+// seek(s, j): the position of node number j of GBWT::sequence(s), i.e. GBWT::start(s) followed by j GBWT::forward steps
+// (src/gbwt.rs:213-229). With checkpoints (cv.table != nullptr) the walk starts from the checkpoint at or before j, at
+// most 2^shift + 31 steps away; without, from start(s). False (and None) when s >= sequences() or j >= the length of s.
+// No walk takes more than walk_limit steps, so a damaged index terminates. `steps` receives the LF steps taken.
+GBWT_HD bool gbwt_seek(const IndexView& ix, const CheckpointView& cv, uint32_t shift, uint64_t s, uint64_t j, gbwt_b200_pos& out,
+                       uint64_t& steps) {
+    set_none(out);
+    steps = 0;
+    if (s >= ix.sequences) return false;
+    gbwt_b200_pos pos;
+    uint64_t at = 0;
+    if (cv.table != nullptr) {
+        if (j >= GBWT_LDG(cv.seq_len + s)) return false;
+        pos = checkpoint_pos(cv, checkpoint_slot(cv, shift, s, j), at);
+    } else if (!gbwt_start(ix, s, pos)) {
+        return false;
+    }
+    for (; at < j; at++) {
+        gbwt_b200_pos next;
+        if (steps >= ix.walk_limit || !gbwt_forward(ix, pos, next)) return false;
+        pos = next;
+        steps++;
+    }
+    out = pos;
+    return true;
+}
+
 }  // namespace gbwt_b200

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../include/gbwt_b200.h"
+#include "../../include/gbwt_b200_ranges.h"
 
 namespace gbwt_b200_host {
 
@@ -155,6 +156,27 @@ public:
         return out;
     }
 
+    // Ranges of sequences (beyond the crate, include/gbwt_b200_ranges.h). seek: the position of node number j of
+    // sequence(seq), nullopt where there is none. sequence_range: sequence(seq)[start .. min(end, len)); dna_range: bytes
+    // [start, min(end, L)) of path_dna(seq) without its endmarker. Both are nullopt iff seq >= sequences(); a start at or
+    // beyond the end gives an empty result.
+    std::optional<Pos> seek(std::size_t seq, std::size_t j) const {
+        uint64_t id = seq, index = j;
+        gbwt_b200_pos out;
+        check(gbwt_b200_seek(h_, &id, &index, 1, &out));
+        return to_pos(out);
+    }
+    std::optional<std::vector<std::size_t>> sequence_range(std::size_t seq, std::size_t start, std::size_t end) const {
+        auto raw = range<uint64_t>(gbwt_b200_extract_ranges, seq, start, end);
+        if (!raw) return std::nullopt;
+        return std::vector<std::size_t>(raw->begin(), raw->end());
+    }
+    std::optional<std::string> dna_range(std::size_t seq, std::size_t start, std::size_t end) const {
+        auto raw = range<uint8_t>(gbwt_b200_extract_dna_ranges, seq, start, end);
+        if (!raw) return std::nullopt;
+        return std::string(raw->begin(), raw->end());
+    }
+
     // Subpath search, src/gbwt.rs:269-304.
     std::optional<SearchState> find(std::size_t node) const {
         uint64_t in = node;
@@ -265,6 +287,18 @@ public:
     }
 
 private:
+    // One range: a call with an empty slot for its length, then one into a slot of that size.
+    template <class T, class Fn>
+    std::optional<std::vector<T>> range(Fn fn, std::size_t seq, std::size_t start, std::size_t end) const {
+        uint64_t id = seq, s = start, e = end, len = 0;
+        const uint64_t none[2] = {0, 0};
+        check(fn(h_, &id, &s, &e, 1, none, nullptr, &len));
+        if (len == UINT64_MAX) return std::nullopt;
+        std::vector<T> out(len);
+        const uint64_t offsets[2] = {0, len};
+        check(fn(h_, &id, &s, &e, 1, offsets, out.data(), &len));
+        return out;
+    }
     std::optional<std::vector<BidirectionalState>> follow(const BidirectionalState& state, int backward) const {
         gbwt_b200_bdstate in{from_state(state.forward), from_state(state.reverse)};
         uint64_t count = 0;
