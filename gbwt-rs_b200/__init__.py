@@ -127,6 +127,8 @@ def _load_library() -> C.CDLL:
         "gbwt_b200_seek_device": (i, [p, p, p, sz, p, p]),
         "gbwt_b200_extract_ranges_device": (i, [p, p, p, p, sz, p, p, p, p]),
         "gbwt_b200_extract_dna_ranges_device": (i, [p, p, p, p, sz, p, p, p, p]),
+        "gbwt_b200_build_image": (i, [p, p, sz, i, i, pp, C.POINTER(sz), p]),
+        "gbwt_b200_build_image_device": (i, [p, p, sz, i, i, p, pp, C.POINTER(sz), p]),
         "gbwt_b200_host_alloc": (p, [sz]), "gbwt_b200_host_free": (None, [p]),
         "gbwt_b200_kernel_launches": (u64, []), "gbwt_b200_version": (C.c_char_p, []),
     }
@@ -263,6 +265,11 @@ class GBWT:
         h = C.c_void_p()
         cls._check(_lib.gbwt_b200_index_from_bytes(_ptr(arr), arr.nbytes, device, _policy(layout, checkpoints, locate), C.byref(h)))
         return cls(h.value)
+
+    @classmethod
+    def build(cls, paths, bidirectional: bool = True, device: int = 0, layout="auto", checkpoints=None, locate=False) -> "GBWT":
+        """The GBWT of the given paths, built on the device (build_image), loaded like from_bytes."""
+        return cls.from_bytes(build_image(paths, bidirectional, device), device, layout, checkpoints, locate)
 
     @classmethod
     def from_parts(cls, sequences, size, offset, alphabet_size, flags, bwt_bytes, record_starts, device: int = 0,
@@ -703,6 +710,60 @@ class GBWT:
 
     def extract_device(self, d_ids: int, m: int, d_out_offsets: int, d_nodes: int, d_lengths: int, stream: int = 0):
         self._check(_lib.gbwt_b200_extract_device(self._h, d_ids, m, d_out_offsets, d_nodes, d_lengths, stream))
+
+
+# ---- building a GBWT from paths (beyond the crate; include/gbwt_b200_build.h) --
+
+def _paths_arrays(paths):
+    """(nodes, offsets) as uint64 arrays from a list of paths or from a (nodes, offsets) pair."""
+    if isinstance(paths, tuple) and len(paths) == 2 and isinstance(paths[1], np.ndarray):
+        return _u64(paths[0]), _u64(paths[1])
+    lengths = [len(p) for p in paths]
+    offsets = np.zeros(len(lengths) + 1, np.uint64)
+    np.cumsum(np.array(lengths, dtype=np.uint64), out=offsets[1:])
+    nodes = np.concatenate([_u64(p) for p in paths]) if offsets[-1] else np.zeros(0, np.uint64)
+    return nodes, offsets
+
+
+def _take_image(call, info):
+    image, n = C.c_void_p(), C.c_size_t(0)
+    stats = np.zeros(4, np.uint64)
+    GBWT._check(call(C.byref(image), C.byref(n), _ptr(stats)))
+    try:
+        out = bytes((C.c_uint8 * n.value).from_address(image.value))
+    finally:
+        _lib.gbwt_b200_free(image)
+    if info is not None:
+        info.update(positions=int(stats[0]), rounds=int(stats[1]), device_us=int(stats[2]), peak_device_bytes=int(stats[3]))
+    return out
+
+
+def build_image(paths, bidirectional: bool = True, device: int = 0, info: Optional[dict] = None) -> bytes:
+    """The Simple-SDS GBWT file of the paths, built on the device: a list of paths (sequences of GBWT node ids) or a
+    (nodes, offsets) pair with path q = nodes[offsets[q]:offsets[q+1]]. bidirectional: sequences 2q = path q and 2q+1 = its
+    reverse with every node flipped. `info`, a dict, receives positions, rounds, device_us and peak_device_bytes."""
+    nodes, offsets = _paths_arrays(paths)
+    n = max(len(offsets) - 1, 0)
+    return _take_image(lambda img, ln, st: _lib.gbwt_b200_build_image(
+        _ptr(nodes) if len(nodes) else None, _ptr(offsets) if len(offsets) else None, n, int(bidirectional), device, img, ln, st), info)
+
+
+def build_image_device(nodes, offsets, n: Optional[int] = None, bidirectional: bool = True, device: int = 0, stream=0,
+                       info: Optional[dict] = None) -> bytes:
+    """build_image from device arrays: torch tensors (int64 / uint64 on the device) or raw addresses, read on `stream`
+    (a torch.cuda.Stream or a cudaStream_t address). Offsets are absolute; n = the number of paths (len(offsets) - 1 for a
+    tensor)."""
+    def addr(x):
+        if hasattr(x, "data_ptr"):
+            if x.element_size() != 8 or not x.is_contiguous():
+                raise ValueError("nodes and offsets must be contiguous 64-bit tensors")
+            return x.data_ptr()
+        return x or None
+    if n is None:
+        n = len(offsets) - 1
+    s = getattr(stream, "cuda_stream", stream) or None
+    return _take_image(lambda img, ln, st: _lib.gbwt_b200_build_image_device(
+        addr(nodes), addr(offsets), n, int(bidirectional), device, s, img, ln, st), info)
 
 
 from .distributed import gather_states, shard_range  # noqa: E402,F401

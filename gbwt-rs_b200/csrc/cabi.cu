@@ -16,7 +16,9 @@
 #include <vector>
 
 #include "../../include/gbwt_b200.h"
+#include "../../include/gbwt_b200_build.h"
 #include "../../include/gbwt_b200_ranges.h"
+#include "build.h"
 #include "find_mixed.h"
 #include "find_window.h"
 #include "kernels.cuh"
@@ -2028,6 +2030,91 @@ int gbwt_b200_node_sequences(const gbwt_b200_index* ix, const uint64_t* node_ids
         return launch_node_sequences(ix, static_cast<uint64_t*>(d[0]), count, static_cast<uint64_t*>(d[2]), out_offsets[q0],
                                      static_cast<uint8_t*>(d[1]), static_cast<uint64_t*>(d[3]), s);
     });
+}
+
+// ---- building a GBWT from paths (gbwt_b200_build.h) ---------------------------------------------------------
+
+static int build_to_image(const uint64_t* d_nodes, const uint64_t* d_offsets, size_t n, int bidirectional, uint64_t extra_bytes,
+                          cudaStream_t s, void** image, size_t* len, uint64_t info[4]) {
+    std::vector<uint8_t> bytes;
+    std::string err;
+    const int rc = build_gbwt_image(d_nodes, d_offsets, n, bidirectional != 0, extra_bytes, s, bytes, info, err);
+    if (rc != GBWT_B200_OK) return fail(rc, err);
+    void* out = std::malloc(std::max<size_t>(bytes.size(), 1));
+    if (out == nullptr) return fail(GBWT_B200_E_IO, "out of memory");
+    std::memcpy(out, bytes.data(), bytes.size());
+    *image = out; *len = bytes.size();
+    return GBWT_B200_OK;
+}
+
+static int check_build_call(int device, void** image, size_t* len, size_t n) {
+    if (image == nullptr || len == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null output");
+    *image = nullptr; *len = 0;
+    if (n == 0) return fail(GBWT_B200_E_ARGUMENT, "no paths");
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
+        cudaGetLastError();
+        return fail(GBWT_B200_E_NO_DEVICE, "no CUDA device available (this library has no CPU fallback)");
+    }
+    if (device < 0 || device >= count) return fail(GBWT_B200_E_ARGUMENT, "invalid device ordinal");
+    return GBWT_B200_OK;
+}
+
+int gbwt_b200_build_image(const uint64_t* nodes, const uint64_t* offsets, size_t n, int bidirectional, int device, void** image,
+                          size_t* len, uint64_t info[4]) {
+    if (int rc = check_build_call(device, image, len, n)) return rc;
+    if (offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null offsets");
+    GBWT_B200_GUARDED(
+        std::string err;
+        uint64_t records = 0;
+        if (int rc = build_check_paths(nodes, offsets, n, bidirectional != 0, records, err)) return fail(rc, err);
+        DeviceScope scope(device);
+        if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
+        const uint64_t path_nodes = offsets[n] - offsets[0];
+        std::vector<uint64_t> rebased(offsets, offsets + n + 1);
+        for (uint64_t& o : rebased) o -= offsets[0];
+        const uint64_t upload = 8 * (path_nodes + n + 1);
+        size_t free_bytes = 0, total_bytes = 0;
+        CUDA_TRY(cudaMemGetInfo(&free_bytes, &total_bytes));
+        const uint64_t need = build_device_bytes(n, path_nodes, bidirectional != 0, records) + upload;
+        if (need > free_bytes)
+            return fail(GBWT_B200_E_CUDA, "the build needs about " + std::to_string(need) + " bytes of device memory; " +
+                                          std::to_string(free_bytes) + " are free");
+        // the copies of the inputs, freed on every path
+        struct Inputs {
+            void* nodes = nullptr;
+            void* offsets = nullptr;
+            cudaStream_t s = nullptr;
+            ~Inputs() { cudaFree(nodes); cudaFree(offsets); if (s) cudaStreamDestroy(s); }
+        } in;
+        CUDA_TRY(cudaStreamCreateWithFlags(&in.s, cudaStreamNonBlocking));
+        CUDA_TRY(cudaMalloc(&in.nodes, std::max<uint64_t>(8 * path_nodes, 8)));
+        CUDA_TRY(cudaMalloc(&in.offsets, 8 * (n + 1)));
+        if (path_nodes > 0) CUDA_TRY(cudaMemcpyAsync(in.nodes, nodes + offsets[0], 8 * path_nodes, cudaMemcpyHostToDevice, in.s));
+        CUDA_TRY(cudaMemcpyAsync(in.offsets, rebased.data(), 8 * (n + 1), cudaMemcpyHostToDevice, in.s));
+        return build_to_image(static_cast<const uint64_t*>(in.nodes), static_cast<const uint64_t*>(in.offsets), n, bidirectional,
+                              upload, in.s, image, len, info);
+    )
+}
+
+int gbwt_b200_build_image_device(const uint64_t* d_nodes, const uint64_t* d_offsets, size_t n, int bidirectional, int device,
+                                 void* stream, void** image, size_t* len, uint64_t info[4]) {
+    if (int rc = check_build_call(device, image, len, n)) return rc;
+    if (d_offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null offsets");
+    GBWT_B200_GUARDED(
+        DeviceScope scope(device);
+        if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
+        // a null d_nodes is refused once the offsets show the paths are not all empty
+        if (d_nodes == nullptr) {
+            uint64_t ends[2] = {0, 0};
+            cudaStream_t s = static_cast<cudaStream_t>(stream);
+            CUDA_TRY(cudaMemcpyAsync(&ends[0], d_offsets, 8, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaMemcpyAsync(&ends[1], d_offsets + n, 8, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaStreamSynchronize(s));
+            if (ends[1] != ends[0]) return fail(GBWT_B200_E_ARGUMENT, "null nodes");
+        }
+        return build_to_image(d_nodes, d_offsets, n, bidirectional, 0, static_cast<cudaStream_t>(stream), image, len, info);
+    )
 }
 
 // ---- utilities ---------------------------------------------------------------------------------------

@@ -11,6 +11,7 @@
 #endif
 
 #include "../../include/gbwt_b200.h"
+#include "record_encode.h"
 
 namespace gbwt_b200 {
 namespace {
@@ -18,26 +19,6 @@ namespace {
 constexpr uint64_t GBWT_TAG = 0x6B376B37ull, GBWT_VERSION = 5;
 constexpr uint64_t FLAG_BIDIRECTIONAL = 1, FLAG_METADATA = 2, FLAG_SIMPLE_SDS = 4;
 constexpr uint64_t GBZ_TAG = 0x205A4247ull, GBZ_VERSION = 2, GRAPH_TAG = 0x6B3764AFull, FLAG_GRAPH_SIMPLE_SDS = 2;
-
-// Either counts or writes: the two passes of the encoder share one code path.
-struct ByteSink {
-    uint8_t* at = nullptr;
-    uint64_t n = 0;
-    void byte(uint8_t b) { if (at != nullptr) at[n] = b; n++; }
-    void varint(uint64_t v) {  // ByteCode::write: 7 bits per byte, least significant first, bit 7 = more to come
-        while (v > 0x7F) { byte(static_cast<uint8_t>((v & 0x7F) | 0x80)); v >>= 7; }
-        byte(static_cast<uint8_t>(v));
-    }
-};
-
-// RLE::write_unchecked for one maximal run.
-void put_run(ByteSink& out, uint64_t sigma, uint64_t value, uint64_t len) {
-    if (sigma >= 255) { out.varint(value); out.varint(len - 1); return; }
-    const uint64_t threshold = 256 / sigma;
-    if (len < threshold) { out.byte(static_cast<uint8_t>(value + sigma * (len - 1))); return; }
-    out.byte(static_cast<uint8_t>(value + sigma * (threshold - 1)));
-    out.varint(len - threshold);
-}
 
 // Feeds the runs of a body to `emit(value, len)` in order (possibly split; the caller merges).
 template <class Emit>
@@ -96,16 +77,10 @@ void put_record(ByteSink& out, const RecordDesc& d, const LayoutArrays& in) {
     if (d.fmt == FMT_EMPTY) { out.varint(0); return; }
     const bool inline_edges = (d.flags & DESC_INLINE_EDGES) != 0;
     const uint64_t sigma = inline_edges ? d.sigma16 : d.w01[1];
-    out.varint(sigma);
-    uint64_t previous = 0;
-    for (uint64_t e = 0; e < sigma; e++) {
-        uint64_t node, offset;
-        if (inline_edges) { node = e == 0 ? d.w01[0] : d.w23[0]; offset = e == 0 ? d.w01[1] : d.w23[1]; }
-        else { node = in.edges[d.w01[0] + e].node; offset = in.edges[d.w01[0] + e].offset; }
-        out.varint(node - previous);
-        out.varint(offset);
-        previous = node;
-    }
+    put_edges(out, sigma, [&](uint64_t e) {
+        if (inline_edges) return e == 0 ? EdgeValue{d.w01[0], d.w01[1]} : EdgeValue{d.w23[0], d.w23[1]};
+        return EdgeValue{in.edges[d.w01[0] + e].node, in.edges[d.w01[0] + e].offset};
+    });
     uint64_t run_value = 0, run_len = 0;
     for_each_run(d, in, [&](uint64_t value, uint64_t len) {
         if (run_len > 0 && value != run_value) { put_run(out, sigma, run_value, run_len); run_len = 0; }
@@ -241,21 +216,26 @@ int write_gbwt_image(const GBWTHeaderFields& header, const LayoutArrays& in, con
     std::vector<uint64_t> starts;
     const int rc = encode_bwt(in, data, starts, err);
     if (rc != GBWT_B200_OK) return rc;
+    write_gbwt_image(header, data.data(), data.size(), starts, carried, image);
+    return GBWT_B200_OK;
+}
+
+void write_gbwt_image(const GBWTHeaderFields& header, const uint8_t* data, uint64_t data_len, const std::vector<uint64_t>& starts,
+                      const Carried& carried, std::vector<uint8_t>& image) {
     image.clear();
-    image.reserve(data.size() + data.size() / 4 + carried.da_samples.size() + carried.metadata.size() + 4096);
+    image.reserve(data_len + data_len / 4 + carried.da_samples.size() + carried.metadata.size() + 4096);
     WordSink w{image};
     const bool has_metadata = carried.metadata.size() > 8;  // Option<Metadata>: more than the size word
     w.word(GBWT_TAG | (GBWT_VERSION << 32));
     w.word(header.sequences); w.word(header.size); w.word(header.offset); w.word(header.alphabet_size);
     w.word((header.flags & FLAG_BIDIRECTIONAL) | FLAG_SIMPLE_SDS | (has_metadata ? FLAG_METADATA : 0));
     put_tags(w, linearize_tags(carried.tags));
-    put_sparse(w, data.size(), starts);
-    w.bytes(data.data(), data.size());
+    put_sparse(w, data_len, starts);
+    w.bytes(data, data_len);
     if (carried.da_samples.empty()) w.word(0);  // an empty Vec<u64>
     else append_bytes(image, carried.da_samples);
     if (!has_metadata) w.word(0);               // Option<Metadata>: None
     else append_bytes(image, carried.metadata);
-    return GBWT_B200_OK;
 }
 
 int write_gbz_image(const GBWTHeaderFields& header, const LayoutArrays& in, const Carried& carried, const uint64_t* label_starts,

@@ -41,6 +41,9 @@ int encode_bwt(const LayoutArrays& in, std::vector<uint8_t>& data, std::vector<u
 // A complete GBWT file image: header, tags, BWT (Elias-Fano index + data), DA samples, Option<Metadata>.
 int write_gbwt_image(const GBWTHeaderFields& header, const LayoutArrays& in, const Carried& carried, std::vector<uint8_t>& image,
                      std::string& err);
+// The same from records already encoded: data[0 .. data_len) with record r at starts[r].
+void write_gbwt_image(const GBWTHeaderFields& header, const uint8_t* data, uint64_t data_len, const std::vector<uint64_t>& starts,
+                      const Carried& carried, std::vector<uint8_t>& image);
 
 // A complete GBZ file image (GBZ::serialize, src/gbz.rs:662-671): header, tags, the GBWT image, the Graph section --
 // the one that was loaded, or (for labels attached with gbwt_b200_index_attach_graph) a version-3 Graph written from

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../include/gbwt_b200.h"
+#include "../../include/gbwt_b200_build.h"
 #include "../../include/gbwt_b200_ranges.h"
 
 namespace gbwt_b200_host {
@@ -68,6 +69,22 @@ public:
         check(gbwt_b200_index_from_parts(sequences, size, offset, alphabet_size, flags, bwt.data(), bwt.size(), record_starts.data(),
                                          record_starts.size(), device, layout, &h));
         return GBWT(h);
+    }
+    // The Simple-SDS GBWT file of the paths, built on the device (gbwt_b200_build.h; beyond the crate, which has no builder).
+    // bidirectional: sequence 2q = path q, 2q+1 = its reverse with every node flipped.
+    static std::vector<uint8_t> build_image(const std::vector<std::vector<uint64_t>>& paths, bool bidirectional = true, int device = 0) {
+        std::vector<uint64_t> nodes, offsets{0};
+        for (const auto& p : paths) { nodes.insert(nodes.end(), p.begin(), p.end()); offsets.push_back(nodes.size()); }
+        void* image = nullptr;
+        std::size_t len = 0;
+        check(gbwt_b200_build_image(nodes.data(), offsets.data(), paths.size(), bidirectional ? 1 : 0, device, &image, &len, nullptr));
+        return take(image, len);
+    }
+    // The GBWT of the paths: build_image loaded with from_bytes.
+    static GBWT build(const std::vector<std::vector<uint64_t>>& paths, bool bidirectional = true, int device = 0,
+                      int layout = GBWT_B200_LAYOUT_AUTO) {
+        const std::vector<uint8_t> image = build_image(paths, bidirectional, device);
+        return from_bytes(image.data(), image.size(), device, layout);
     }
     // serialize::serialize_to (src/gbwt.rs:388-400): the Simple-SDS GBWT file, tags, DA samples and metadata as loaded.
     void save(const std::string& path) const { check(gbwt_b200_index_save_file(h_, path.c_str())); }
