@@ -129,6 +129,8 @@ def _load_library() -> C.CDLL:
         "gbwt_b200_extract_dna_ranges_device": (i, [p, p, p, p, sz, p, p, p, p]),
         "gbwt_b200_build_image": (i, [p, p, sz, i, i, pp, C.POINTER(sz), p]),
         "gbwt_b200_build_image_device": (i, [p, p, sz, i, i, p, pp, C.POINTER(sz), p]),
+        "gbwt_b200_insert_image": (i, [p, p, p, sz, pp, C.POINTER(sz), p]),
+        "gbwt_b200_insert_image_device": (i, [p, p, p, sz, p, pp, C.POINTER(sz), p]),
         "gbwt_b200_host_alloc": (p, [sz]), "gbwt_b200_host_free": (None, [p]),
         "gbwt_b200_kernel_launches": (u64, []), "gbwt_b200_version": (C.c_char_p, []),
     }
@@ -270,6 +272,29 @@ class GBWT:
     def build(cls, paths, bidirectional: bool = True, device: int = 0, layout="auto", checkpoints=None, locate=False) -> "GBWT":
         """The GBWT of the given paths, built on the device (build_image), loaded like from_bytes."""
         return cls.from_bytes(build_image(paths, bidirectional, device), device, layout, checkpoints, locate)
+
+    # -- inserting paths (beyond the crate; include/gbwt_b200_insert.h) --
+    def insert_image(self, paths, info: Optional[dict] = None) -> bytes:
+        """The Simple-SDS GBWT file of this index's sequences followed by the paths (a list of paths or a (nodes, offsets)
+        pair), equal to build_image(<this index's paths> + paths, bidirectional=self.is_bidirectional()). The index is
+        not modified. `info` receives positions, rounds, device_us, peak_device_bytes, longest and walk_us."""
+        nodes, offsets = _paths_arrays(paths)
+        n = max(len(offsets) - 1, 0)
+        return _take_image(lambda img, ln, st: _lib.gbwt_b200_insert_image(
+            self._h, _ptr(nodes) if len(nodes) else None, _ptr(offsets) if len(offsets) else None, n, img, ln, st), info, insert=True)
+
+    def insert_image_device(self, nodes, offsets, n: Optional[int] = None, stream=0, info: Optional[dict] = None) -> bytes:
+        """insert_image from device arrays on this index's device: torch tensors (int64 / uint64) or raw addresses, read on
+        `stream`. Offsets are absolute. Merging index B into this one: B.extract_device(...) output as nodes / offsets."""
+        if n is None:
+            n = len(offsets) - 1
+        s = getattr(stream, "cuda_stream", stream) or None
+        return _take_image(lambda img, ln, st: _lib.gbwt_b200_insert_image_device(
+            self._h, _device_addr(nodes), _device_addr(offsets), n, s, img, ln, st), info, insert=True)
+
+    def insert(self, paths, layout="auto", checkpoints=None, locate=False) -> "GBWT":
+        """A new index: insert_image(paths) loaded with from_bytes on this index's device. This index is unchanged."""
+        return type(self).from_bytes(self.insert_image(paths), self.device(), layout, checkpoints, locate)
 
     @classmethod
     def from_parts(cls, sequences, size, offset, alphabet_size, flags, bwt_bytes, record_starts, device: int = 0,
@@ -725,9 +750,9 @@ def _paths_arrays(paths):
     return nodes, offsets
 
 
-def _take_image(call, info):
+def _take_image(call, info, insert=False):
     image, n = C.c_void_p(), C.c_size_t(0)
-    stats = np.zeros(4, np.uint64)
+    stats = np.zeros(6, np.uint64)
     GBWT._check(call(C.byref(image), C.byref(n), _ptr(stats)))
     try:
         out = bytes((C.c_uint8 * n.value).from_address(image.value))
@@ -735,7 +760,17 @@ def _take_image(call, info):
         _lib.gbwt_b200_free(image)
     if info is not None:
         info.update(positions=int(stats[0]), rounds=int(stats[1]), device_us=int(stats[2]), peak_device_bytes=int(stats[3]))
+        if insert:
+            info.update(longest=int(stats[4]), walk_us=int(stats[5]))
     return out
+
+
+def _device_addr(x):
+    if hasattr(x, "data_ptr"):
+        if x.element_size() != 8 or not x.is_contiguous():
+            raise ValueError("nodes and offsets must be contiguous 64-bit tensors")
+        return x.data_ptr()
+    return x or None
 
 
 def build_image(paths, bidirectional: bool = True, device: int = 0, info: Optional[dict] = None) -> bytes:
@@ -753,17 +788,11 @@ def build_image_device(nodes, offsets, n: Optional[int] = None, bidirectional: b
     """build_image from device arrays: torch tensors (int64 / uint64 on the device) or raw addresses, read on `stream`
     (a torch.cuda.Stream or a cudaStream_t address). Offsets are absolute; n = the number of paths (len(offsets) - 1 for a
     tensor)."""
-    def addr(x):
-        if hasattr(x, "data_ptr"):
-            if x.element_size() != 8 or not x.is_contiguous():
-                raise ValueError("nodes and offsets must be contiguous 64-bit tensors")
-            return x.data_ptr()
-        return x or None
     if n is None:
         n = len(offsets) - 1
     s = getattr(stream, "cuda_stream", stream) or None
     return _take_image(lambda img, ln, st: _lib.gbwt_b200_build_image_device(
-        addr(nodes), addr(offsets), n, int(bidirectional), device, s, img, ln, st), info)
+        _device_addr(nodes), _device_addr(offsets), n, int(bidirectional), device, s, img, ln, st), info)
 
 
 from .distributed import gather_states, shard_range  # noqa: E402,F401

@@ -15,9 +15,9 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libgbwt_b200.so")
-SOURCES = [os.path.join(CSRC, f) for f in ("cabi.cu", "find_mixed.cu", "find_window.cu", "layout_builder.cpp", "sds_loader.cpp", "layout_writer.cpp", "locate.cu", "ranges.cu", "build.cu")]
-HEADERS = [os.path.join(CSRC, f) for f in ("kernels.cuh", "find_lean.cuh", "find_mixed.h", "find_window.h", "record_scan.cuh", "layout.h", "layout_builder.h", "sds_loader.h", "layout_writer.h", "locate.h", "ranges.h", "build.h", "record_encode.h")] + \
-          [os.path.join(os.path.dirname(HERE), "include", f) for f in ("gbwt_b200.h", "gbwt_b200_ranges.h", "gbwt_b200_build.h")]
+SOURCES = [os.path.join(CSRC, f) for f in ("cabi.cu", "find_mixed.cu", "find_window.cu", "layout_builder.cpp", "sds_loader.cpp", "layout_writer.cpp", "locate.cu", "ranges.cu", "build.cu", "insert.cu")]
+HEADERS = [os.path.join(CSRC, f) for f in ("kernels.cuh", "find_lean.cuh", "find_mixed.h", "find_window.h", "record_scan.cuh", "layout.h", "layout_builder.h", "sds_loader.h", "layout_writer.h", "locate.h", "ranges.h", "build.h", "record_encode.h", "insert.h", "insert_step.h")] + \
+          [os.path.join(os.path.dirname(HERE), "include", f) for f in ("gbwt_b200.h", "gbwt_b200_ranges.h", "gbwt_b200_build.h", "gbwt_b200_insert.h")]
 
 
 def nvcc_path() -> str:

@@ -59,15 +59,6 @@ __device__ __forceinline__ uint64_t lower_bound(const T* __restrict__ a, uint64_
     return lo;
 }
 
-// Sequence s: its first position in the expanded array and its length.
-struct SeqSpan { uint64_t start, len; };
-__device__ __forceinline__ SeqSpan seq_span(const uint64_t* __restrict__ offsets, uint64_t s, bool bidirectional) {
-    const uint64_t q = bidirectional ? s >> 1 : s, base = offsets[0];
-    const uint64_t lo = offsets[q] - base, len = offsets[q + 1] - offsets[q];
-    if (!bidirectional) return {lo, len};
-    return {2 * lo + (s & 1) * len, len};
-}
-
 __global__ void __launch_bounds__(BUILD_THREADS) k_build_check_offsets(const uint64_t* __restrict__ offsets, uint64_t n,
                                                                        BuildStats* __restrict__ stats) {
     for (uint64_t q = first_index(); q < n; q += stride())
@@ -324,35 +315,6 @@ __global__ void __launch_bounds__(BUILD_THREADS) k_build_write_runs(const uint32
     }
 }
 
-// Device scratch with a byte count: every block is freed when the scratch goes out of scope.
-struct Scratch {
-    std::vector<std::pair<void*, uint64_t>> blocks;
-    uint64_t live = 0, peak = 0;
-    ~Scratch() { for (auto& b : blocks) cudaFree(b.first); }
-    template <class T>
-    cudaError_t get(T*& p, uint64_t count) {
-        const uint64_t bytes = std::max<uint64_t>(count * sizeof(T), 16);
-        void* raw = nullptr;
-        const cudaError_t e = cudaMalloc(&raw, bytes);
-        p = static_cast<T*>(raw);
-        if (e != cudaSuccess) return e;
-        blocks.emplace_back(raw, bytes);
-        live += bytes;
-        peak = std::max(peak, live);
-        return cudaSuccess;
-    }
-    void drop(const void* p) {
-        if (p == nullptr) return;
-        for (size_t i = 0; i < blocks.size(); i++) {
-            if (blocks[i].first != p) continue;
-            cudaFree(blocks[i].first);
-            live -= blocks[i].second;
-            blocks.erase(blocks.begin() + static_cast<std::ptrdiff_t>(i));
-            return;
-        }
-    }
-};
-
 int bits_for(uint64_t v) {  // bits needed for every value below v
     int b = 0;
     while (b < 64 && (v - 1) >> b) b++;
@@ -400,20 +362,25 @@ uint64_t build_device_bytes(uint64_t paths, uint64_t path_nodes, bool bidirectio
     return 36 * entries + 28 * (records + 1) + (uint64_t(64) << 20);
 }
 
-int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_t n, bool bidirectional, uint64_t extra_bytes,
-                     cudaStream_t s, std::vector<uint8_t>& image, uint64_t* info, std::string& err) {
-    cudaError_t ce = cudaSuccess;
+// ---- the phases (build.h) ----------------------------------------------------------------------------------
+
 #define BUILD_TRY(expr)                                                                              \
     do {                                                                                             \
-        ce = (expr);                                                                                 \
-        if (ce != cudaSuccess) { err = std::string(#expr) + ": " + cudaGetErrorString(ce); return GBWT_B200_E_CUDA; } \
+        const cudaError_t ce_ = (expr);                                                              \
+        if (ce_ != cudaSuccess) { err = std::string(#expr) + ": " + cudaGetErrorString(ce_); return GBWT_B200_E_CUDA; } \
     } while (0)
-    int device = 0, sm_count = 0;
+
+int device_sm_count(int& sm_count, std::string& err) {
+    int device = 0;
     BUILD_TRY(cudaGetDevice(&device));
     BUILD_TRY(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, device));
-    Scratch scratch;
-    const auto t0 = std::chrono::steady_clock::now();
+    return GBWT_B200_OK;
+}
 
+int build_sort(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_t n, bool bidirectional, const ExtraNeed& extra, bool keep_rank,
+               int sm_count, cudaStream_t s, Scratch& scratch, SortedPaths& sp, std::string& err) {
+    sp = SortedPaths{};
+    sp.n = n; sp.bidirectional = bidirectional;
     // ---- checks, read back before any working memory is taken ----
     BuildStats* d_stats = nullptr;
     BUILD_TRY(scratch.get(d_stats, 1));
@@ -437,8 +404,11 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
         if (int rc = status_of(h_stats.flags, err)) return rc;
     }
     const uint64_t N = bidirectional ? 2 * n : n, T = bidirectional ? 2 * path_nodes : path_nodes, M = N + T;
-    const uint64_t offset = T > 0 ? h_stats.min_node - 1 : 0, alphabet_size = T > 0 ? uint64_t(h_stats.max_node) + 1 : 1;
-    const uint64_t records = alphabet_size - offset;
+    sp.path_nodes = path_nodes; sp.N = N; sp.T = T; sp.M = M;
+    sp.offset = T > 0 ? h_stats.min_node - 1 : 0;
+    sp.alphabet_size = T > 0 ? uint64_t(h_stats.max_node) + 1 : 1;
+    sp.records = sp.alphabet_size - sp.offset;
+    const uint64_t records = sp.records;
     const int bits = bits_for(M);
     size_t sort_bytes = 0, scan_bytes = 0;
     if (T > 0) {
@@ -451,34 +421,32 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
     {
         size_t free_bytes = 0, total_bytes = 0;
         BUILD_TRY(cudaMemGetInfo(&free_bytes, &total_bytes));
-        const uint64_t need = build_device_bytes(n, path_nodes, bidirectional, records) + temp_bytes;
+        const uint64_t need = build_device_bytes(n, path_nodes, bidirectional, records) + temp_bytes + (extra.bytes ? extra.bytes(sp) : 0);
         if (need > free_bytes) {
-            err = "the build needs about " + std::to_string(need) + " bytes of device memory; " + std::to_string(free_bytes) + " are free";
+            err = std::string("the ") + extra.what + " needs about " + std::to_string(need) + " bytes of device memory; " +
+                  std::to_string(free_bytes) + " are free";
             return GBWT_B200_E_CUDA;
         }
     }
 
     // ---- prefix doubling over the T positions ----
-    uint32_t* order = nullptr;  // the final order of the positions
-    uint32_t *sym = nullptr, *seq = nullptr;
-    uint64_t rounds = 0;
     if (T > 0) {
         uint32_t *rank = nullptr, *pos[2] = {nullptr, nullptr};
         uint64_t* keys[2] = {nullptr, nullptr};
-        BUILD_TRY(scratch.get(sym, T));
-        BUILD_TRY(scratch.get(seq, T));
+        BUILD_TRY(scratch.get(sp.sym, T));
+        BUILD_TRY(scratch.get(sp.seq, T));
         BUILD_TRY(scratch.get(rank, T));
         for (int b = 0; b < 2; b++) { BUILD_TRY(scratch.get(keys[b], T)); BUILD_TRY(scratch.get(pos[b], T)); }
         cub::DoubleBuffer<uint64_t> kb(keys[0], keys[1]);
         cub::DoubleBuffer<uint32_t> pb(pos[0], pos[1]);
         uint8_t* temp = nullptr;
         BUILD_TRY(scratch.get(temp, temp_bytes));
-        k_build_expand<<<grid_of(path_nodes, sm_count), BUILD_THREADS, 0, s>>>(d_nodes, d_offsets, n, path_nodes, bidirectional, sym, seq);
+        k_build_expand<<<grid_of(path_nodes, sm_count), BUILD_THREADS, 0, s>>>(d_nodes, d_offsets, n, path_nodes, bidirectional, sp.sym, sp.seq);
         BUILD_TRY(cudaGetLastError());
         const unsigned grid = grid_of(T, sm_count);
         for (uint64_t h = 0;; h = h == 0 ? 1 : 2 * h) {
-            if (h == 0) k_build_symbol_keys<<<grid, BUILD_THREADS, 0, s>>>(sym, T, kb.Current(), pb.Current());
-            else k_build_keys<<<grid, BUILD_THREADS, 0, s>>>(rank, seq, T, h, bits, kb.Current(), pb.Current());
+            if (h == 0) k_build_symbol_keys<<<grid, BUILD_THREADS, 0, s>>>(sp.sym, T, kb.Current(), pb.Current());
+            else k_build_keys<<<grid, BUILD_THREADS, 0, s>>>(rank, sp.seq, T, h, bits, kb.Current(), pb.Current());
             BUILD_TRY(cudaGetLastError());
             size_t tb = temp_bytes;
             BUILD_TRY(cub::DeviceRadixSort::SortPairs(temp, tb, kb, pb, static_cast<uint32_t>(T), 0,
@@ -493,28 +461,38 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
             uint32_t groups = 0;
             BUILD_TRY(cudaMemcpyAsync(&groups, group + T - 1, 4, cudaMemcpyDeviceToHost, s));
             BUILD_TRY(cudaStreamSynchronize(s));
-            if (h > 0) rounds++;
+            if (h > 0) sp.rounds++;
             if (groups == T) break;
         }
-        order = pb.Current();
-        scratch.drop(temp); scratch.drop(rank); scratch.drop(pb.Alternate());
+        sp.order = pb.Current();
+        scratch.drop(temp); scratch.drop(pb.Alternate());
         scratch.drop(keys[0]); scratch.drop(keys[1]);
+        if (keep_rank) sp.rank = rank; else scratch.drop(rank);
     }
+    scratch.drop(d_stats);
+    return GBWT_B200_OK;
+}
 
-    // ---- entries, records, edges ----
-    uint32_t *rec = nullptr, *value = nullptr, *pred = nullptr, *rec_first = nullptr;
-    BUILD_TRY(scratch.get(rec, M));
-    BUILD_TRY(scratch.get(value, M));
-    BUILD_TRY(scratch.get(pred, M));
-    BUILD_TRY(scratch.get(rec_first, records + 1));
+int build_entries_edges(SortedPaths& sp, const uint64_t* d_offsets, int sm_count, cudaStream_t s, Scratch& scratch, BuiltEdges& be,
+                        std::string& err) {
+    be = BuiltEdges{};
+    const uint64_t N = sp.N, T = sp.T, M = sp.M, offset = sp.offset, records = sp.records;
+    BuildStats* d_stats = nullptr;
+    BUILD_TRY(scratch.get(d_stats, 1));
+    BUILD_TRY(scratch.get(be.rec, M));
+    BUILD_TRY(scratch.get(be.value, M));
+    BUILD_TRY(scratch.get(be.pred, M));
+    BUILD_TRY(scratch.get(be.rec_first, records + 1));
+    uint32_t *rec = be.rec, *value = be.value, *pred = be.pred;
     const unsigned grid = grid_of(M, sm_count);
-    k_build_entries<<<grid, BUILD_THREADS, 0, s>>>(order, sym, seq, d_offsets, N, T, bidirectional, offset, rec, value, pred);
+    k_build_entries<<<grid, BUILD_THREADS, 0, s>>>(sp.order, sp.sym, sp.seq, d_offsets, N, T, sp.bidirectional, offset, rec, value, pred);
     BUILD_TRY(cudaGetLastError());
-    scratch.drop(order); scratch.drop(sym); scratch.drop(seq);
-    k_build_record_firsts<<<grid_of(records + 1, sm_count), BUILD_THREADS, 0, s>>>(rec, M, 0, records + 1, rec_first);
+    scratch.drop(sp.order); scratch.drop(sp.sym); scratch.drop(sp.seq);
+    sp.order = sp.sym = sp.seq = nullptr;
+    k_build_record_firsts<<<grid_of(records + 1, sm_count), BUILD_THREADS, 0, s>>>(rec, M, 0, records + 1, be.rec_first);
     BUILD_TRY(cudaGetLastError());
     BUILD_TRY(cudaMemsetAsync(&d_stats->count, 0, 8, s));
-    k_build_edges<<<grid, BUILD_THREADS, 0, s>>>(rec, value, pred, rec_first, N, M, offset, d_stats, nullptr, nullptr);
+    k_build_edges<<<grid, BUILD_THREADS, 0, s>>>(rec, value, pred, be.rec_first, N, M, offset, d_stats, nullptr, nullptr);
     BUILD_TRY(cudaGetLastError());
     unsigned long long raw_edges = 0;
     BUILD_TRY(cudaMemcpyAsync(&raw_edges, &d_stats->count, 8, cudaMemcpyDeviceToHost, s));
@@ -523,11 +501,8 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
     uint32_t* eoffs[2] = {nullptr, nullptr};
     for (int b = 0; b < 2; b++) { BUILD_TRY(scratch.get(ekeys[b], raw_edges)); BUILD_TRY(scratch.get(eoffs[b], raw_edges)); }
     BUILD_TRY(cudaMemsetAsync(&d_stats->count, 0, 8, s));
-    k_build_edges<<<grid, BUILD_THREADS, 0, s>>>(rec, value, pred, rec_first, N, M, offset, d_stats, ekeys[0], eoffs[0]);
+    k_build_edges<<<grid, BUILD_THREADS, 0, s>>>(rec, value, pred, be.rec_first, N, M, offset, d_stats, ekeys[0], eoffs[0]);
     BUILD_TRY(cudaGetLastError());
-    uint64_t edges = 0;
-    uint64_t* edge_keys = nullptr;
-    uint32_t* edge_offs = nullptr;
     {
         cub::DoubleBuffer<uint64_t> kb(ekeys[0], ekeys[1]);
         cub::DoubleBuffer<uint32_t> ob(eoffs[0], eoffs[1]);
@@ -548,19 +523,26 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
         unsigned long long selected = 0;
         BUILD_TRY(cudaMemcpyAsync(&selected, d_selected, 8, cudaMemcpyDeviceToHost, s));
         BUILD_TRY(cudaStreamSynchronize(s));
-        edges = selected;
-        edge_keys = kb.Alternate(); edge_offs = ob.Alternate();
+        be.edges = selected;
+        be.edge_keys = kb.Alternate(); be.edge_offs = ob.Alternate();
         scratch.drop(temp); scratch.drop(kb.Current()); scratch.drop(ob.Current());
     }
-    uint32_t* edge_first = nullptr;
-    BUILD_TRY(scratch.get(edge_first, records + 1));
-    k_build_record_firsts<<<grid_of(records + 1, sm_count), BUILD_THREADS, 0, s>>>(edge_keys, edges, 32, records + 1, edge_first);
+    BUILD_TRY(scratch.get(be.edge_first, records + 1));
+    k_build_record_firsts<<<grid_of(records + 1, sm_count), BUILD_THREADS, 0, s>>>(be.edge_keys, be.edges, 32, records + 1, be.edge_first);
     BUILD_TRY(cudaGetLastError());
-    k_build_values<<<grid, BUILD_THREADS, 0, s>>>(rec, value, M, edge_first, edge_keys);
+    k_build_values<<<grid, BUILD_THREADS, 0, s>>>(rec, value, M, be.edge_first, be.edge_keys);
     BUILD_TRY(cudaGetLastError());
+    scratch.drop(d_stats);
+    return GBWT_B200_OK;
+}
 
-    // ---- runs and bytes ----
-    uint32_t* heads = pred;  // the predecessors are done with
+int build_write_records(const SortedPaths& sp, BuiltEdges& be, int sm_count, cudaStream_t s, Scratch& scratch, std::vector<uint8_t>& h_data,
+                        std::vector<uint64_t>& h_starts, std::string& err) {
+    const uint64_t M = sp.M, records = sp.records;
+    const uint32_t *rec = be.rec, *value = be.value, *rec_first = be.rec_first, *edge_first = be.edge_first, *edge_offs = be.edge_offs;
+    const uint64_t* edge_keys = be.edge_keys;
+    const unsigned grid = grid_of(M, sm_count);
+    uint32_t* heads = be.pred;  // the predecessors are done with
     k_build_run_heads<<<grid, BUILD_THREADS, 0, s>>>(rec, value, M, heads);
     BUILD_TRY(cudaGetLastError());
     uint64_t runs = 0;
@@ -580,7 +562,8 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
         BUILD_TRY(scratch.get(run_start, runs + 1));
         k_build_run_starts<<<grid, BUILD_THREADS, 0, s>>>(rec, value, heads, M, run_start);
         BUILD_TRY(cudaGetLastError());
-        scratch.drop(pred);
+        scratch.drop(be.pred);
+        be.pred = nullptr;
     }
     BUILD_TRY(scratch.get(run_off, runs + 1));
     BUILD_TRY(scratch.get(rec_start, records + 1));
@@ -613,20 +596,37 @@ int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_
     BUILD_TRY(cudaGetLastError());
     k_build_write_runs<<<grid_of(runs, sm_count), BUILD_THREADS, 0, s>>>(run_start, runs, rec, value, edge_first, run_off, run_base, data);
     BUILD_TRY(cudaGetLastError());
-    std::vector<uint8_t> h_data(data_len);
-    std::vector<uint64_t> h_starts(records);
+    h_data.resize(data_len);
+    h_starts.resize(records);
     if (data_len > 0) BUILD_TRY(cudaMemcpyAsync(h_data.data(), data, data_len, cudaMemcpyDeviceToHost, s));
     BUILD_TRY(cudaMemcpyAsync(h_starts.data(), rec_start, records * 8, cudaMemcpyDeviceToHost, s));
     BUILD_TRY(cudaStreamSynchronize(s));
-    const uint64_t device_us = std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
-#undef BUILD_TRY
-
-    GBWTHeaderFields header;
-    header.sequences = N; header.size = M; header.offset = offset; header.alphabet_size = alphabet_size;
-    header.flags = bidirectional ? 1 : 0;
-    write_gbwt_image(header, h_data.data(), data_len, h_starts, Carried{}, image);
-    if (info != nullptr) { info[0] = M; info[1] = rounds; info[2] = device_us; info[3] = scratch.peak + extra_bytes; }
     return GBWT_B200_OK;
 }
+
+int build_gbwt_image(const uint64_t* d_nodes, const uint64_t* d_offsets, uint64_t n, bool bidirectional, uint64_t extra_bytes,
+                     cudaStream_t s, std::vector<uint8_t>& image, uint64_t* info, std::string& err) {
+    int sm_count = 0;
+    if (int rc = device_sm_count(sm_count, err)) return rc;
+    Scratch scratch;
+    const auto t0 = std::chrono::steady_clock::now();
+    SortedPaths sp;
+    BuiltEdges be;
+    std::vector<uint8_t> h_data;
+    std::vector<uint64_t> h_starts;
+    if (int rc = build_sort(d_nodes, d_offsets, n, bidirectional, ExtraNeed{}, false, sm_count, s, scratch, sp, err)) return rc;
+    if (int rc = build_entries_edges(sp, d_offsets, sm_count, s, scratch, be, err)) return rc;
+    if (int rc = build_write_records(sp, be, sm_count, s, scratch, h_data, h_starts, err)) return rc;
+    const uint64_t device_us = std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
+
+    GBWTHeaderFields header;
+    header.sequences = sp.N; header.size = sp.M; header.offset = sp.offset; header.alphabet_size = sp.alphabet_size;
+    header.flags = bidirectional ? 1 : 0;
+    write_gbwt_image(header, h_data.data(), h_data.size(), h_starts, Carried{}, image);
+    if (info != nullptr) { info[0] = sp.M; info[1] = sp.rounds; info[2] = device_us; info[3] = scratch.peak + extra_bytes; }
+    return GBWT_B200_OK;
+}
+
+#undef BUILD_TRY
 
 }  // namespace gbwt_b200

@@ -11,16 +11,19 @@
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
+#include <functional>
 #include <string>
 #include <type_traits>
 #include <vector>
 
 #include "../../include/gbwt_b200.h"
 #include "../../include/gbwt_b200_build.h"
+#include "../../include/gbwt_b200_insert.h"
 #include "../../include/gbwt_b200_ranges.h"
 #include "build.h"
 #include "find_mixed.h"
 #include "find_window.h"
+#include "insert.h"
 #include "kernels.cuh"
 #include "layout_builder.h"
 #include "layout_writer.h"
@@ -2060,40 +2063,66 @@ static int check_build_call(int device, void** image, size_t* len, size_t n) {
     return GBWT_B200_OK;
 }
 
+// Host paths on the current device for a build or an insertion: the checks of build_check_paths, the memory check (`need`
+// from the records and the bytes of the copies), then the copies on a new stream, freed on every path.
+struct PathUpload {
+    void* nodes = nullptr;
+    void* offsets = nullptr;
+    cudaStream_t s = nullptr;
+    uint64_t bytes = 0;
+    PathUpload() = default;
+    PathUpload(const PathUpload&) = delete;
+    PathUpload& operator=(const PathUpload&) = delete;
+    ~PathUpload() { cudaFree(nodes); cudaFree(offsets); if (s) cudaStreamDestroy(s); }
+};
+
+static int upload_paths(const uint64_t* nodes, const uint64_t* offsets, size_t n, bool bidirectional, const char* what,
+                        const std::function<uint64_t(uint64_t, uint64_t)>& need_of, PathUpload& in) {
+    std::string err;
+    uint64_t records = 0;
+    if (int rc = build_check_paths(nodes, offsets, n, bidirectional, records, err)) return fail(rc, err);
+    const uint64_t path_nodes = offsets[n] - offsets[0];
+    std::vector<uint64_t> rebased(offsets, offsets + n + 1);
+    for (uint64_t& o : rebased) o -= offsets[0];
+    in.bytes = 8 * (path_nodes + n + 1);
+    size_t free_bytes = 0, total_bytes = 0;
+    CUDA_TRY(cudaMemGetInfo(&free_bytes, &total_bytes));
+    const uint64_t need = need_of(path_nodes, records) + in.bytes;
+    if (need > free_bytes)
+        return fail(GBWT_B200_E_CUDA, std::string("the ") + what + " needs about " + std::to_string(need) + " bytes of device memory; " +
+                                      std::to_string(free_bytes) + " are free");
+    CUDA_TRY(cudaStreamCreateWithFlags(&in.s, cudaStreamNonBlocking));
+    CUDA_TRY(cudaMalloc(&in.nodes, std::max<uint64_t>(8 * path_nodes, 8)));
+    CUDA_TRY(cudaMalloc(&in.offsets, 8 * (n + 1)));
+    if (path_nodes > 0) CUDA_TRY(cudaMemcpyAsync(in.nodes, nodes + offsets[0], 8 * path_nodes, cudaMemcpyHostToDevice, in.s));
+    CUDA_TRY(cudaMemcpyAsync(in.offsets, rebased.data(), 8 * (n + 1), cudaMemcpyHostToDevice, in.s));
+    return GBWT_B200_OK;
+}
+
+// A null d_nodes is refused once the offsets show the paths are not all empty.
+static int check_device_nodes(const uint64_t* d_nodes, const uint64_t* d_offsets, size_t n, cudaStream_t s) {
+    if (d_nodes != nullptr) return GBWT_B200_OK;
+    uint64_t ends[2] = {0, 0};
+    CUDA_TRY(cudaMemcpyAsync(&ends[0], d_offsets, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(&ends[1], d_offsets + n, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    if (ends[1] != ends[0]) return fail(GBWT_B200_E_ARGUMENT, "null nodes");
+    return GBWT_B200_OK;
+}
+
 int gbwt_b200_build_image(const uint64_t* nodes, const uint64_t* offsets, size_t n, int bidirectional, int device, void** image,
                           size_t* len, uint64_t info[4]) {
     if (int rc = check_build_call(device, image, len, n)) return rc;
     if (offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null offsets");
     GBWT_B200_GUARDED(
-        std::string err;
-        uint64_t records = 0;
-        if (int rc = build_check_paths(nodes, offsets, n, bidirectional != 0, records, err)) return fail(rc, err);
         DeviceScope scope(device);
         if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
-        const uint64_t path_nodes = offsets[n] - offsets[0];
-        std::vector<uint64_t> rebased(offsets, offsets + n + 1);
-        for (uint64_t& o : rebased) o -= offsets[0];
-        const uint64_t upload = 8 * (path_nodes + n + 1);
-        size_t free_bytes = 0, total_bytes = 0;
-        CUDA_TRY(cudaMemGetInfo(&free_bytes, &total_bytes));
-        const uint64_t need = build_device_bytes(n, path_nodes, bidirectional != 0, records) + upload;
-        if (need > free_bytes)
-            return fail(GBWT_B200_E_CUDA, "the build needs about " + std::to_string(need) + " bytes of device memory; " +
-                                          std::to_string(free_bytes) + " are free");
-        // the copies of the inputs, freed on every path
-        struct Inputs {
-            void* nodes = nullptr;
-            void* offsets = nullptr;
-            cudaStream_t s = nullptr;
-            ~Inputs() { cudaFree(nodes); cudaFree(offsets); if (s) cudaStreamDestroy(s); }
-        } in;
-        CUDA_TRY(cudaStreamCreateWithFlags(&in.s, cudaStreamNonBlocking));
-        CUDA_TRY(cudaMalloc(&in.nodes, std::max<uint64_t>(8 * path_nodes, 8)));
-        CUDA_TRY(cudaMalloc(&in.offsets, 8 * (n + 1)));
-        if (path_nodes > 0) CUDA_TRY(cudaMemcpyAsync(in.nodes, nodes + offsets[0], 8 * path_nodes, cudaMemcpyHostToDevice, in.s));
-        CUDA_TRY(cudaMemcpyAsync(in.offsets, rebased.data(), 8 * (n + 1), cudaMemcpyHostToDevice, in.s));
+        PathUpload in;
+        if (int rc = upload_paths(nodes, offsets, n, bidirectional != 0, "build", [&](uint64_t path_nodes, uint64_t records) {
+                return build_device_bytes(n, path_nodes, bidirectional != 0, records);
+            }, in)) return rc;
         return build_to_image(static_cast<const uint64_t*>(in.nodes), static_cast<const uint64_t*>(in.offsets), n, bidirectional,
-                              upload, in.s, image, len, info);
+                              in.bytes, in.s, image, len, info);
     )
 }
 
@@ -2104,16 +2133,66 @@ int gbwt_b200_build_image_device(const uint64_t* d_nodes, const uint64_t* d_offs
     GBWT_B200_GUARDED(
         DeviceScope scope(device);
         if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
-        // a null d_nodes is refused once the offsets show the paths are not all empty
-        if (d_nodes == nullptr) {
-            uint64_t ends[2] = {0, 0};
-            cudaStream_t s = static_cast<cudaStream_t>(stream);
-            CUDA_TRY(cudaMemcpyAsync(&ends[0], d_offsets, 8, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(cudaMemcpyAsync(&ends[1], d_offsets + n, 8, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(cudaStreamSynchronize(s));
-            if (ends[1] != ends[0]) return fail(GBWT_B200_E_ARGUMENT, "null nodes");
-        }
+        if (int rc = check_device_nodes(d_nodes, d_offsets, n, static_cast<cudaStream_t>(stream))) return rc;
         return build_to_image(d_nodes, d_offsets, n, bidirectional, 0, static_cast<cudaStream_t>(stream), image, len, info);
+    )
+}
+
+// ---- inserting paths into an index (gbwt_b200_insert.h) ----------------------------------------------------------
+
+static InsertTarget insert_target(const gbwt_b200_index* ix) {
+    InsertTarget a;
+    a.view = ix->view;
+    a.size = ix->size;
+    a.edges_total = ix->edges_total;
+    a.body_bytes = ix->bytes[1];
+    return a;
+}
+
+static int insert_to_image(const gbwt_b200_index* ix, const uint64_t* d_nodes, const uint64_t* d_offsets, size_t n, uint64_t extra_bytes,
+                           cudaStream_t s, void** image, size_t* len, uint64_t info[6]) {
+    std::vector<uint8_t> bytes;
+    std::string err;
+    const int rc = insert_gbwt_image(insert_target(ix), d_nodes, d_offsets, n, extra_bytes, s, bytes, info, err);
+    if (rc != GBWT_B200_OK) return fail(rc, err);
+    void* out = std::malloc(std::max<size_t>(bytes.size(), 1));
+    if (out == nullptr) return fail(GBWT_B200_E_IO, "out of memory");
+    std::memcpy(out, bytes.data(), bytes.size());
+    *image = out; *len = bytes.size();
+    return GBWT_B200_OK;
+}
+
+static int check_insert_call(const gbwt_b200_index* ix, void** image, size_t* len, size_t n) {
+    if (int rc = check_index(ix)) return rc;
+    return check_build_call(ix->device, image, len, n);
+}
+
+int gbwt_b200_insert_image(const gbwt_b200_index* ix, const uint64_t* nodes, const uint64_t* offsets, size_t n, void** image, size_t* len,
+                           uint64_t info[6]) {
+    if (int rc = check_insert_call(ix, image, len, n)) return rc;
+    if (offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null offsets");
+    GBWT_B200_GUARDED(
+        DeviceScope scope(ix->device);
+        if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
+        const bool bidirectional = (ix->flags & GBWT_FLAG_BIDIRECTIONAL) != 0;
+        PathUpload in;
+        if (int rc = upload_paths(nodes, offsets, n, bidirectional, "insertion", [&](uint64_t path_nodes, uint64_t) {
+                return build_device_bytes(n, path_nodes, bidirectional, 1);
+            }, in)) return rc;
+        return insert_to_image(ix, static_cast<const uint64_t*>(in.nodes), static_cast<const uint64_t*>(in.offsets), n, in.bytes, in.s,
+                               image, len, info);
+    )
+}
+
+int gbwt_b200_insert_image_device(const gbwt_b200_index* ix, const uint64_t* d_nodes, const uint64_t* d_offsets, size_t n, void* stream,
+                                  void** image, size_t* len, uint64_t info[6]) {
+    if (int rc = check_insert_call(ix, image, len, n)) return rc;
+    if (d_offsets == nullptr) return fail(GBWT_B200_E_ARGUMENT, "null offsets");
+    GBWT_B200_GUARDED(
+        DeviceScope scope(ix->device);
+        if (!scope.ok) return fail(GBWT_B200_E_CUDA, "cudaSetDevice failed");
+        if (int rc = check_device_nodes(d_nodes, d_offsets, n, static_cast<cudaStream_t>(stream))) return rc;
+        return insert_to_image(ix, d_nodes, d_offsets, n, 0, static_cast<cudaStream_t>(stream), image, len, info);
     )
 }
 

@@ -20,58 +20,6 @@ constexpr uint64_t GBWT_TAG = 0x6B376B37ull, GBWT_VERSION = 5;
 constexpr uint64_t FLAG_BIDIRECTIONAL = 1, FLAG_METADATA = 2, FLAG_SIMPLE_SDS = 4;
 constexpr uint64_t GBZ_TAG = 0x205A4247ull, GBZ_VERSION = 2, GRAPH_TAG = 0x6B3764AFull, FLAG_GRAPH_SIMPLE_SDS = 2;
 
-// Feeds the runs of a body to `emit(value, len)` in order (possibly split; the caller merges).
-template <class Emit>
-void for_each_run(const RecordDesc& d, const LayoutArrays& in, Emit emit) {
-    const uint8_t* body = reinterpret_cast<const uint8_t*>(in.bodies + 2 * static_cast<uint64_t>(d.body));
-    switch (d.fmt) {
-    case FMT_SINGLE:
-        if (d.total_len > 0) emit(0, d.total_len);
-        break;
-    case FMT_DENSE2: {
-        const uint32_t* words = reinterpret_cast<const uint32_t*>(body);
-        uint64_t run_value = 0, run_len = 0;
-        for (uint64_t i = 0; i < d.total_len; i++) {
-            const uint64_t blk = i / DENSE_BITS, bit = i % DENSE_BITS;
-            const uint64_t v = (words[blk * 8 + 2 + bit / 32] >> (bit % 32)) & 1u;
-            if (run_len > 0 && v != run_value) { emit(run_value, run_len); run_len = 0; }
-            run_value = v; run_len++;
-        }
-        if (run_len > 0) emit(run_value, run_len);
-        break;
-    }
-    case FMT_DENSE4: {
-        const uint32_t* words = reinterpret_cast<const uint32_t*>(body);
-        uint64_t run_value = 0, run_len = 0;
-        for (uint64_t i = 0; i < d.total_len; i++) {
-            const uint64_t blk = i / DENSE4_POSITIONS, at = i % DENSE4_POSITIONS;
-            const uint64_t v = (words[blk * 8 + 4 + at / 16] >> (2 * (at % 16))) & 3u;
-            if (run_len > 0 && v != run_value) { emit(run_value, run_len); run_len = 0; }
-            run_value = v; run_len++;
-        }
-        if (run_len > 0) emit(run_value, run_len);
-        break;
-    }
-    case FMT_RUN8: {
-        const uint64_t sigma = (d.flags & DESC_INLINE_EDGES) ? d.sigma16 : d.w01[1];
-        for (uint64_t i = 0; i < d.body_len; i++) emit(body[i] % sigma, body[i] / sigma + 1);
-        break;
-    }
-    case FMT_RUN32: {
-        const uint32_t* w = reinterpret_cast<const uint32_t*>(body);
-        for (uint64_t i = 0; i < d.body_len; i++) emit(w[i] & 0xFFu, static_cast<uint64_t>(w[i] >> 8) + 1);
-        break;
-    }
-    case FMT_RUN64: {
-        const uint32_t* w = reinterpret_cast<const uint32_t*>(body);
-        for (uint64_t i = 0; i < d.body_len; i++) emit(w[2 * i], w[2 * i + 1]);
-        break;
-    }
-    default:
-        break;
-    }
-}
-
 // One record in the encoding of BWTBuilder::append: sigma, (node delta, offset) per edge, maximal runs.
 void put_record(ByteSink& out, const RecordDesc& d, const LayoutArrays& in) {
     if (d.fmt == FMT_EMPTY) { out.varint(0); return; }
@@ -82,7 +30,7 @@ void put_record(ByteSink& out, const RecordDesc& d, const LayoutArrays& in) {
         return EdgeValue{in.edges[d.w01[0] + e].node, in.edges[d.w01[0] + e].offset};
     });
     uint64_t run_value = 0, run_len = 0;
-    for_each_run(d, in, [&](uint64_t value, uint64_t len) {
+    for_each_run(d, in.bodies, [&](uint64_t value, uint64_t len) {
         if (run_len > 0 && value != run_value) { put_run(out, sigma, run_value, run_len); run_len = 0; }
         run_value = value; run_len += len;
     });

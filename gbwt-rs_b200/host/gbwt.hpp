@@ -86,6 +86,21 @@ public:
         const std::vector<uint8_t> image = build_image(paths, bidirectional, device);
         return from_bytes(image.data(), image.size(), device, layout);
     }
+    // The Simple-SDS GBWT file of this index's sequences followed by the paths, inserted on the device (gbwt_b200_insert.h;
+    // beyond the crate): build_image(<this index's paths> + paths) with this index's orientation. This index is unchanged.
+    std::vector<uint8_t> insert_image(const std::vector<std::vector<uint64_t>>& paths) const {
+        std::vector<uint64_t> nodes, offsets{0};
+        for (const auto& p : paths) { nodes.insert(nodes.end(), p.begin(), p.end()); offsets.push_back(nodes.size()); }
+        void* image = nullptr;
+        std::size_t len = 0;
+        check(gbwt_b200_insert_image(h_, nodes.data(), offsets.data(), paths.size(), &image, &len, nullptr));
+        return take(image, len);
+    }
+    // A new index: insert_image loaded with from_bytes on this index's device.
+    GBWT insert(const std::vector<std::vector<uint64_t>>& paths, int layout = GBWT_B200_LAYOUT_AUTO) const {
+        const std::vector<uint8_t> image = insert_image(paths);
+        return from_bytes(image.data(), image.size(), gbwt_b200_device(h_), layout);
+    }
     // serialize::serialize_to (src/gbwt.rs:388-400): the Simple-SDS GBWT file, tags, DA samples and metadata as loaded.
     void save(const std::string& path) const { check(gbwt_b200_index_save_file(h_, path.c_str())); }
     std::vector<uint8_t> serialize() const {

@@ -23,12 +23,14 @@
  * Limits of this version:
  *  - ranks are 32 bits: nodes + sequences must be below 2^32;
  *  - device memory: about 36 bytes per position (nodes + sequences) and 28 bytes per record, plus the sort's temporary
- *    storage. A path set that does not fit is refused; there is no external or merged construction.
+ *    storage. A path set that does not fit is refused; it can be built in pieces by inserting paths into a loaded index
+ *    (gbwt_b200_insert.h, included here).
  */
 #ifndef GBWT_B200_BUILD_H
 #define GBWT_B200_BUILD_H
 
 #include "gbwt_b200.h"
+#include "gbwt_b200_insert.h"
 
 #ifdef __cplusplus
 extern "C" {
